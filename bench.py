@@ -9,8 +9,9 @@ random initial states and controls (SURVEY.md 8d), strong-scaled: the B problems
 one process per GPU, no collective on the solve path (torch.distributed is used for the timing barrier and the
 final reduction of counters only).
 A "step" is one pass of the iLQG loop (derivative kernel, backward-pass kernel, line-search kernel) over the rank's
-whole shard; K steps = a solve with max_iter = K.  W warm-up steps run first on the same inputs (a throw-away
-solve with max_iter = W).  `value` = (line searches performed by all problems on all ranks) / (max over ranks of
+whole shard; K steps = a solve with max_iter = K, which makes K passes unless every problem of the shard has stopped before
+(`passes` in the JSON line is the number made; fewer than K is also reported on stderr).  W warm-up steps run first on the
+same inputs (a throw-away solve with max_iter = W).  `value` = (line searches performed by all problems on all ranks) / (max over ranks of
 the device time of the K timed steps incl. the initial rollout), inputs resident in HBM.  `e2e` = the same count
 over the time of ONE call of the public C ABI's end-to-end entry (ilqgb_solve_host): upload (pinned host -> HBM) + solve +
 download of x, u, cost, iterations (HBM -> pinned host), pipelined per chunk stream.  The iteration count follows SURVEY.md 8d: loop passes that reached line_search.
@@ -25,6 +26,13 @@ the surveyed max_iter = 50.  Each carries a bit-exactness flag against the CPU r
 the process exit non-zero after the JSON line is printed.
 
 `--gpus N` without torchrun (WORLD_SIZE unset) drives N GPUs from this one process through ilqgb_create_multi.
+
+`--dump-outputs DIR` writes what the end-to-end leg's call returned after its last timed step (the same results as the
+resident leg: the run checks the costs of both bit for bit), as float64 .npy files in DIR:
+cost.npy, iterations.npy, result.npy, n_linesearch.npy of every problem (a seeded sample of 2^19 problems above that batch) with
+their problem numbers in problem_index.npy, and the trajectories x.npy [n][T+1][4] and u.npy [n][T][2] of a seeded sample of 1024
+problems (traj_index.npy); under 64 MB at any batch.  The inputs are a fixed function of the problem number, so two builds run with
+the same arguments can be compared output for output.
 
 `--impl reference` times the reference's own C solver (oracle/_ref, the unmodified sources compiled -O3
 -ffp-contract=off; falls back to the oracle port if that library is not present) on all host cores, one solver
@@ -152,6 +160,24 @@ def make_inputs(first, count, pinned):
         a, b = W.car_batch(n, T=T_HOR, first=first + s)
         x0[s:s + n] = a
         u0[s:s + n] = b
+
+
+DUMP_PROBLEMS, DUMP_TRAJECTORIES = 1 << 19, 1024
+
+
+def dump_outputs(path, x, u, cost, iterations, result, n_linesearch):
+    """The arrays a caller of the timed solve receives, as float64 .npy files; samples are seeded and depend on the batch only."""
+    os.makedirs(path, exist_ok=True)
+    B = cost.shape[0]
+
+    def sample(n):
+        return np.arange(B) if B <= n else np.sort(np.random.default_rng(0).choice(B, size=n, replace=False))
+
+    pi, ti = sample(DUMP_PROBLEMS), sample(DUMP_TRAJECTORIES)
+    arrays = {"problem_index": pi, "cost": cost[pi], "iterations": iterations[pi], "result": result[pi], "n_linesearch": n_linesearch[pi],
+              "traj_index": ti, "x": x[ti], "u": u[ti]}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 def cpu_reference_run(n_problems, max_iter, threads, first=0, problem=PROBLEM, ddp=FULL_DDP, inputs=None, params=None):
@@ -409,6 +435,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the other BASELINE configs (config 3, config 5, config 4 at max_iter=50)")
     ap.add_argument("--chunks", type=int, default=0, help="concurrent streams per GPU (0 = automatic)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed solve returned as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -425,6 +452,8 @@ def main():
 
     import ilqg_b200
 
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs needs the whole batch in one process (--gpus N without torchrun drives N GPUs)")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py (impl=ours) needs a CUDA device: the solver has no CPU path")
     torch.cuda.set_device(local_rank)
@@ -513,6 +542,8 @@ def main():
     S.download_ptr(None, None, cost_out.data_ptr(), it_out.data_ptr(), res_out.data_ptr(), nls_out.data_ptr())
     n_ls = int(nls_out.numpy().sum())
     cost_resident = cost_out.numpy().copy()
+    # passes of the iLQG loop the timed solve made: --steps unless every problem of the shard stopped earlier
+    passes = int(reduce(int(it_out.numpy().max()), dist.ReduceOp.MAX if world > 1 else None))
 
     ms_max = reduce(ms_dev, dist.ReduceOp.MAX if world > 1 else None)
     its_total = reduce(n_ls, dist.ReduceOp.SUM if world > 1 else None)
@@ -537,6 +568,8 @@ def main():
     sampler.stop()
     n_ls_e2e = int(nls_out.numpy().sum())
     deterministic = bool(np.array_equal(cost_resident, cost_out.numpy()))
+    if args.dump_outputs:   # the host buffers hold what this leg's call returned; no copy beyond the timed one
+        dump_outputs(args.dump_outputs, x_out.numpy(), u_out.numpy(), cost_out.numpy(), it_out.numpy(), res_out.numpy(), nls_out.numpy())
     ms_e2e_max = reduce(ms_e2e, dist.ReduceOp.MAX if world > 1 else None)
     its_e2e = reduce(n_ls_e2e, dist.ReduceOp.SUM if world > 1 else None)
     h2d = x0_t.numel() * 8 + u0_t.numel() * 8
@@ -597,7 +630,7 @@ def main():
 
     if rank == 0:
         line = {
-            "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": n_gpus, "steps": args.steps, "warmup": args.warmup,
+            "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": n_gpus, "steps": args.steps, "passes": passes, "warmup": args.warmup,
             "ms_per_step": ms_max / max(args.steps, 1), "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
             "dtype": "f64", "data": "synthetic", "config": workload_config(args), "clocks": clocks,
             "e2e": {"value": its_e2e / (ms_e2e_max * 1e-3), "unit": UNIT, "h2d_bytes_per_step": h2d_tot / max(args.steps, 1),
@@ -611,6 +644,8 @@ def main():
         }
         print(json.dumps(line))
         sys.stdout.flush()
+        if passes < args.steps:
+            sys.stderr.write(f"bench.py: every problem stopped after {passes} of the {args.steps} passes --steps allows\n")
     if S is not None:
         S.close()
     if world > 1:

@@ -1,7 +1,8 @@
-"""The reference's OWN example problem files (examples/CarParking/optDefCar.mac, examples/Brachistochrone/optDefBrachi.mac,
-optDefBrachi_hli.mac) through the one-step build `python -m ilqg_gen.make file.mac`: the resulting product libraries solve on the
-GPU bit-exactly like the unmodified reference core linked against the C generated from the same file.  The libraries are built
-where /root/reference exists (__graft_entry__.build_mac_examples) and travel to the GPU box prebuilt."""
+"""The reference's example problems (CarParking, Brachistochrone, Brachistochrone with hli), restated as problem files in
+tests/data/, through the one-step build `python -m ilqg_gen.make file.mac`: the resulting product libraries solve on the GPU
+bit-exactly like the solver core linked against the C generated from the same file -- the unmodified reference core where it
+was built against that C, else the oracle port, which reproduces the reference's golden fixtures bit for bit
+(test_oracle_golden.py).  __graft_entry__.build() builds the libraries and their checkers (build_mac_examples)."""
 import os
 
 import numpy as np
@@ -13,6 +14,7 @@ from ilqg_b200 import workloads as W
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MAC_LIB = os.path.join(ROOT, "ddp-generator_b200", "build_mac", "lib")
+MAC_PROBLEMS = os.path.join(ROOT, "ddp-generator_b200", "build_mac", "problems")
 GOLD = os.path.join(ROOT, "tests", "golden")
 
 
@@ -27,15 +29,23 @@ def _case(name):
     return 120, params, x0[None], u0[None], opts
 
 
+def _checker(name, ddp):
+    """The reference core where its library is at least as new as the C generated from tests/data/<name>.mac (an older one was
+    linked against the C of another problem file and is not rebuilt without the reference's sources), else the oracle port."""
+    ref, gen = oracle_lib.lib_path("reference", name, ddp), os.path.join(MAC_PROBLEMS, name, "iLQG_func.c")
+    fresh = os.path.exists(ref) and os.path.exists(gen) and os.path.getmtime(ref) >= os.path.getmtime(gen)
+    return "reference" if fresh else "port"
+
+
 def _have(name, ddp):
-    return os.path.exists(ilqg_b200.lib_path(name, ddp, MAC_LIB)) and oracle_lib.available("reference", name, ddp)
+    return os.path.exists(ilqg_b200.lib_path(name, ddp, MAC_LIB)) and oracle_lib.available(_checker(name, ddp), name, ddp)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["mac_car", "mac_brachi", "mac_brachi_hli"])
 @pytest.mark.parametrize("ddp", [0, 1])
 def test_mac_built_library_matches_reference_core(name, ddp):
-    assert _have(name, ddp), "build the .mac examples first: python -c 'import __graft_entry__ as g; g.build()' where /root/reference exists"
+    assert _have(name, ddp), "build the .mac examples first: python -c 'import __graft_entry__ as g; g.build()'"
     T, params, x0, u0, opts = _case(name)
     s = ilqg_b200.BatchSolver(name, ddp, x0.shape[0], T, flags=ilqg_b200.TRACE, lib_dir=MAC_LIB)
     s.set_options(opts); s.set_params(params)
@@ -43,7 +53,7 @@ def test_mac_built_library_matches_reference_core(name, ddp):
     tr_a, tr_l = s.get_int("tr_alpha"), s.get("tr_lambda")
     mu_f = s.get("mu_f") if name != "mac_car" else None
     s.close()
-    O = oracle_lib.OracleLib("reference", name, ddp)
+    O = oracle_lib.OracleLib(_checker(name, ddp), name, ddp)
     for b in range(x0.shape[0]):
         h = O.solver(T); h.set_opts(opts); h.set_params(params)
         assert h.init(x0[b], u0[b])
@@ -61,14 +71,14 @@ def test_mac_built_library_matches_reference_core(name, ddp):
 @pytest.mark.parametrize("name,fixture,T", [("mac_brachi", "brachi_n500_ddp0.npz", 500), ("mac_brachi_hli", "brachi_hli_ddp0.npz", 500),
                                             ("mac_car", "car_T100_b0.npz", 100)])
 def test_mac_model_agrees_with_the_handwritten_module(name, fixture, T):
-    """CPU: the reference core on the C generated from the .mac file reaches the solution the fixtures hold (which were recorded
-    with the hand-written problem modules).  The two front ends may order floating-point operations differently, so the first
-    pass is compared to 1e-12 relative and -- for the Brachistochrone, which is not chaotic -- the final cost to 1e-9."""
-    if not oracle_lib.available("reference", name, 0):
-        pytest.skip("reference core / .mac examples not built on this machine")
+    """CPU: the solver core (the reference's where it is built, else the oracle port) on the C generated from the .mac file
+    reaches the solution the fixtures hold (which were recorded with the hand-written problem modules).  The two front ends may
+    order floating-point operations differently, so the first pass is compared to 1e-12 relative and -- for the Brachistochrone,
+    which is not chaotic -- the final cost to 1e-9."""
+    assert oracle_lib.available(_checker(name, 0), name, 0), "build the .mac examples first: python -c 'import __graft_entry__ as g; g.build()'"
     g = np.load(os.path.join(GOLD, fixture))
     params, opts = {"mac_car": (W.CAR_PARAMS, {"max_iter": 30.0}), "mac_brachi": W.brachi(T)[0::3], "mac_brachi_hli": W.brachi_hli(T)[0::3]}[name]
-    h = oracle_lib.OracleLib("reference", name, 0).solver(T)
+    h = oracle_lib.OracleLib(_checker(name, 0), name, 0).solver(T)
     h.set_opts(opts); h.set_params(params)
     assert h.init(g["x0"], g["u0"])
     assert abs(h.scalar("cost") - float(g["cost0"])) <= 1e-12 * abs(float(g["cost0"]))
