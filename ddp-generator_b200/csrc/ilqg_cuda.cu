@@ -96,6 +96,7 @@ int ilqgk_preload(void)
     bad |= preload_pp<false>() | preload_pp<true>();
     bad |= split_launcher<P, false, SPLIT_OK>::preload() | split_launcher<P, true, SPLIT_OK>::preload();
     bad |= preload_one(k_finalize) | preload_one(k_count_active) | preload_one(k_scatter) | preload_one(k_gather);
+    bad |= preload_one(k_mpc_advance<P>);   /* first launched between two steps of a closed loop, while other chunks solve */
     if (bad) { snprintf(g_err, sizeof g_err, "loading the kernels failed: %s", cudaGetErrorString(cudaGetLastError())); return -1; }
     if (dev >= 0 && dev < ILQGK_MAX_DEVICES) loaded[dev] = 1;
     return 0;
@@ -343,6 +344,12 @@ int ilqgk_launch_count_active(const ilqg_work *w, int *d_counter, void *stream)
     if (check(cudaMemsetAsync(d_counter, 0, sizeof(int), (cudaStream_t)stream), "memset")) return -1;
     k_count_active<<<nblk(w->B, 256), 256, 0, (cudaStream_t)stream>>>(*w, d_counter);
     return check(cudaGetLastError(), "k_count_active");
+}
+
+int ilqgk_launch_mpc_advance(const ilqg_work *w, const ilqg_mpc_step *a, void *stream)
+{
+    k_mpc_advance<P><<<nblk(w->B, 256), 256, 0, (cudaStream_t)stream>>>(*w, *a);
+    return check(cudaGetLastError(), "k_mpc_advance");
 }
 
 int ilqgk_launch_scatter(const double *src, double *dst, double *dst_alt, const int *sel, int B, int n_k, int n_i, long long stride_k,

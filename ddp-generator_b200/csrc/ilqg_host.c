@@ -45,7 +45,8 @@ struct chunk {
     /* asynchronous solve engine (run_engine): progress polls in flight, early stop, gating */
     int *h_poll;           /* pinned ring of POLL_RING running-problem counts */
     void *ev_poll[4];
-    int poll_issued, poll_seen, stop, phase;
+    int poll_issued, poll_seen, stop, phase, mpc_step;
+    ilqg_mpc_step mpc;     /* closed loop (ilqgb_mpc): this chunk's step and its w / log arrays in the staging buffer */
     void *ev_gate;
     int gate_recorded;
     int ls_tail_from;      /* -1 = choose by batch size */
@@ -570,6 +571,99 @@ static int ck_upload(chunk *h, const double *x0, const double *u_nom)
     h->n_launches += 2;
     if (ilqgk_launch_scatter(h->d_stage + B * T * nu, h->w.x0, NULL, NULL, h->B, 1, h->d.nx, 0, 1, h->Bp, 0, h->stream)) return failk(h);
     h->started = 0;
+    return 0;
+}
+
+/* ---- receding horizon -------------------------------------------------------------------------------------------------------- */
+/* the solution becomes the next solve's input: controls shifted by n_shift, x0 from the host or x[n_shift] (+ w [B][nx]) */
+static int ck_shift(chunk *h, int n_shift, const double *x0, const double *w)
+{
+    const size_t B = (size_t)h->B, nx = (size_t)h->d.nx;
+    ilqg_mpc_step a;
+    if (ilqgk_set_device(h->device)) return failk(h);
+    if ((x0 || w) && ensure_stage(h, B * nx)) return -1;
+    memset(&a, 0, sizeof a);
+    a.n_shift = n_shift;
+    a.set_x0 = !x0;
+    a.plan = 1;
+    a.n_steps = 1;
+    if (w) {
+        if (ilqgk_h2d(h->d_stage, w, sizeof(double) * B * nx, h->stream)) return failk(h);
+        a.w = h->d_stage;
+    }
+    if (ilqgk_launch_mpc_advance(&h->w, &a, h->stream)) return failk(h);
+    h->n_launches++;
+    if (x0) { /* into its own [NX][Bp] array, as ck_upload does */
+        if (ilqgk_h2d(h->d_stage, x0, sizeof(double) * B * nx, h->stream)) return failk(h);
+        if (ilqgk_launch_scatter(h->d_stage, h->w.x0, NULL, NULL, h->B, 1, h->d.nx, 0, 1, h->Bp, 0, h->stream)) return failk(h);
+        h->n_launches++;
+    }
+    h->started = 0;
+    return 0;
+}
+
+/* a closed loop of n_steps (ilqgb_mpc): host w [B][n_steps][nx] (may be NULL) and log arrays (any may be NULL) of the caller */
+typedef struct {
+    int n_steps;
+    const double *w;
+    double *x, *u, *cost;
+    int *iterations, *result;
+} mpc_t;
+
+/* w and the logs of one closed loop live in the staging buffer, problem-major, so that they go to and from the caller's
+   arrays in one copy each; w (the chunk's slice) is uploaded here */
+static int ck_mpc_begin(chunk *h, const mpc_t *m, const double *w)
+{
+    const size_t B = (size_t)h->B, S = (size_t)m->n_steps, nx = (size_t)h->d.nx, nu = (size_t)h->d.nu, ints = (B * S + 1) / 2;
+    const size_t n_w = w ? B * S * nx : 0, n_x = m->x ? B * (S + 1) * nx : 0, n_u = m->u ? B * S * nu : 0, n_c = m->cost ? B * S : 0;
+    const size_t n_it = m->iterations ? ints : 0, n_res = m->result ? ints : 0;
+    double *s;
+    if (ilqgk_set_device(h->device)) return failk(h);
+    if (ensure_stage(h, n_w + n_x + n_u + n_c + n_it + n_res)) return -1;
+    s = h->d_stage;
+    memset(&h->mpc, 0, sizeof h->mpc);
+    h->mpc.n_shift = 1;
+    h->mpc.set_x0 = 1;
+    h->mpc.n_steps = m->n_steps;
+    if (w) {
+        if (ilqgk_h2d(s, w, sizeof(double) * n_w, h->stream)) return failk(h);
+        h->mpc.w = s;
+    }
+    s += n_w;
+    h->mpc.x_log = m->x ? s : NULL;
+    s += n_x;
+    h->mpc.u_log = m->u ? s : NULL;
+    s += n_u;
+    h->mpc.cost_log = m->cost ? s : NULL;
+    s += n_c;
+    h->mpc.it_log = m->iterations ? (int *)s : NULL;
+    s += n_it;
+    h->mpc.res_log = m->result ? (int *)s : NULL;
+    return 0;
+}
+
+/* after the solve of step `step`: log it; unless it was the last one, its solution becomes the next step's input */
+static int ck_mpc_advance(chunk *h, int step)
+{
+    h->mpc.step = step;
+    h->mpc.plan = step + 1 < h->mpc.n_steps;
+    if (ilqgk_launch_mpc_advance(&h->w, &h->mpc, h->stream)) return failk(h);
+    h->n_launches++;
+    if (h->mpc.plan) h->started = 0;   /* the input has been replaced */
+    return 0;
+}
+
+/* the chunk's logs into the caller's arrays (problem `first` of the handle is row 0 of this chunk) */
+static int ck_mpc_logs(chunk *h, const mpc_t *m, size_t first)
+{
+    const size_t B = (size_t)h->B, S = (size_t)m->n_steps, nx = (size_t)h->d.nx, nu = (size_t)h->d.nu;
+    const ilqg_mpc_step *a = &h->mpc;
+    if (ilqgk_set_device(h->device)) return failk(h);
+    if (m->x && ilqgk_d2h(m->x + first * (S + 1) * nx, a->x_log, sizeof(double) * B * (S + 1) * nx, h->stream)) return failk(h);
+    if (m->u && ilqgk_d2h(m->u + first * S * nu, a->u_log, sizeof(double) * B * S * nu, h->stream)) return failk(h);
+    if (m->cost && ilqgk_d2h(m->cost + first * S, a->cost_log, sizeof(double) * B * S, h->stream)) return failk(h);
+    if (m->iterations && ilqgk_d2h(m->iterations + first * S, a->it_log, sizeof(int) * B * S, h->stream)) return failk(h);
+    if (m->result && ilqgk_d2h(m->result + first * S, a->res_log, sizeof(int) * B * S, h->stream)) return failk(h);
     return 0;
 }
 
@@ -1352,7 +1446,7 @@ static int engine_poll(chunk *c)
     return 0;
 }
 
-static int run_engine(ilqgb_handle *h, const io_t *io)
+static int run_engine(ilqgb_handle *h, const io_t *io, const mpc_t *mpc)
 {
     int i, remaining, rc = 0;
     const int prio = io && h->e2e_prio && h->n > 1;
@@ -1369,8 +1463,9 @@ static int run_engine(ilqgb_handle *h, const io_t *io)
     }
     for (i = 0; i < h->n; i++) {
         chunk *c = h->c[i];
-        c->poll_issued = c->poll_seen = c->stop = c->phase = c->gate_recorded = 0;
+        c->poll_issued = c->poll_seen = c->stop = c->phase = c->gate_recorded = c->mpc_step = 0;
         if (io && ck_upload(c, io->x0 + (size_t)h->first[i] * h->d.nx, io->u_nom + (size_t)h->first[i] * h->T * h->d.nu)) { rc = hfail(h, c); goto out; }
+        if (mpc && ck_mpc_begin(c, mpc, mpc->w ? mpc->w + (size_t)h->first[i] * mpc->n_steps * h->d.nx : NULL)) { rc = hfail(h, c); goto out; }
     }
     remaining = h->n;
     while (remaining > 0) {
@@ -1417,6 +1512,17 @@ static int run_engine(ilqgb_handle *h, const io_t *io)
                 }
                 if (ilqgk_launch_finalize(&c->w, max_iter, c->stream)) { rc = hfail(h, NULL); goto out; }
                 c->n_launches++;
+                if (mpc) { /* closed loop: log the step and, until the last one, solve again from the shifted solution */
+                    if (ck_mpc_advance(c, c->mpc_step)) { rc = hfail(h, c); goto out; }
+                    progressed = 1;
+                    if (++c->mpc_step < mpc->n_steps) {
+                        /* polls still in flight belong to the finished solve: a zero among them must not stop the next one.
+                           They are dropped; their slots are recorded again before they are read. */
+                        c->poll_issued = c->poll_seen = c->stop = 0;
+                        c->phase = 0;
+                        continue;
+                    }
+                }
                 if (io) {
                     const size_t f = (size_t)h->first[i];
                     if (ck_download_async(c, io->x ? io->x + f * (h->T + 1) * h->d.nx : NULL, io->u ? io->u + f * h->T * h->d.nu : NULL,
@@ -1430,6 +1536,9 @@ static int run_engine(ilqgb_handle *h, const io_t *io)
         }
         if (!progressed) nanosleep(&nap, NULL);
     }
+    if (mpc) /* the logs of every chunk, once all of them have finished their last step */
+        for (i = 0; i < h->n; i++)
+            if (ck_mpc_logs(h->c[i], mpc, (size_t)h->first[i])) { rc = hfail(h, h->c[i]); goto out; }
 out:
     if (join_streams(h)) rc = -1;
     if (prio) {
@@ -1439,7 +1548,7 @@ out:
     return rc;
 }
 
-int ilqgb_solve(ilqgb_handle *h) { return run_engine(h, NULL); }
+int ilqgb_solve(ilqgb_handle *h) { return run_engine(h, NULL, NULL); }
 
 /* End to end from and to host buffers (pinned for full overlap); same results as upload + solve + download. */
 int ilqgb_solve_host(ilqgb_handle *h, const double *x0, const double *u_nom, double *x, double *u, double *cost,
@@ -1447,7 +1556,41 @@ int ilqgb_solve_host(ilqgb_handle *h, const double *x0, const double *u_nom, dou
 {
     io_t io = {x0, u_nom, x, u, cost, iterations, result, n_linesearch};
     if (!x0 || !u_nom) { snprintf(h->err, sizeof h->err, "x0 and u_nom are required"); return -1; }
-    if (run_engine(h, &io)) return -1;
+    if (run_engine(h, &io, NULL)) return -1;
+    return ilqgb_sync(h);
+}
+
+/* Receding horizon (the reference's caller shifts u between two iLQG_mex calls; SURVEY.md:211): see ilqg_b200.h */
+int ilqgb_shift(ilqgb_handle *h, int n_shift, const double *x0, const double *w)
+{
+    int i;
+    if (n_shift < 0 || n_shift > h->T) { snprintf(h->err, sizeof h->err, "n_shift must be in 0..n_hor"); return -1; }
+    if (x0 && w) { snprintf(h->err, sizeof h->err, "w is added to the solution's state: it cannot go with x0"); return -1; }
+    for (i = 0; i < h->n; i++)
+        if (!h->c[i]->started) { snprintf(h->err, sizeof h->err, "ilqgb_start has not been called since the last upload or shift"); return -1; }
+    if (fork_streams(h)) return -1;
+    for (i = 0; i < h->n; i++) {
+        const size_t f = (size_t)h->first[i] * h->d.nx;
+        if (ck_shift(h->c[i], n_shift, x0 ? x0 + f : NULL, w ? w + f : NULL)) return hfail(h, h->c[i]);
+    }
+    return join_streams(h);
+}
+
+/* Every chunk runs its own closed loop in the solve engine: when a solve of the chunk finishes, k_mpc_advance logs it and
+   shifts it into the next input, and the chunk starts again at once -- a chunk that converged early does not wait for the
+   others, which a host loop of ilqgb_shift + ilqgb_solve would make it do at every step. */
+int ilqgb_mpc(ilqgb_handle *h, int n_steps, const double *x0, const double *u_nom, const double *w, double *x_cl, double *u_cl,
+              double *cost, int *iterations, int *result)
+{
+    const mpc_t m = {n_steps, w, x_cl, u_cl, cost, iterations, result};
+    int i;
+    if (n_steps < 1) { snprintf(h->err, sizeof h->err, "n_steps must be >= 1"); return -1; }
+    if (!x0 != !u_nom) { snprintf(h->err, sizeof h->err, "x0 and u_nom go together (neither: continue from the current input)"); return -1; }
+    if (!x0)
+        for (i = 0; i < h->n; i++)
+            if (h->c[i]->started) { snprintf(h->err, sizeof h->err, "no input to continue from: ilqgb_upload or ilqgb_shift since the last start"); return -1; }
+    if (x0 && ilqgb_upload(h, x0, u_nom)) return -1;
+    if (run_engine(h, NULL, &m)) return -1;
     return ilqgb_sync(h);
 }
 

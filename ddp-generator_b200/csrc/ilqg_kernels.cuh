@@ -2085,6 +2085,65 @@ __global__ void k_count_active(Work w, int *out)
     if (threadIdx.x == 0 && a) atomicAdd(out, a);
 }
 
+/* Receding horizon (ilqgb_shift / ilqgb_mpc), one thread per problem: log the finished solve (its x0, the applied control
+ * u[0], cost, iterations, result), then make its solution the input of the next solve, which is what the reference's caller
+ * does between two iLQG_mex calls: the shifted controls go into the u part of buffer 0's records, where ilqgb_upload puts
+ * them and k_init's initial rollout reads them, and x[n_shift] (+ w) becomes x0.  Whatever the nominal buffer holds is
+ * used, also for a problem whose solve failed.  When cur[b] == 0 the source is the destination: every record is read before
+ * it is written because the steps are copied in ascending order, KB of them loaded before any is stored (a copy parallel
+ * over (k, b) would not be safe).  Adjacent threads are adjacent problems of the [k][Bp][RXU] records. */
+template <class P>
+__global__ void __launch_bounds__(256) k_mpc_advance(Work w, ilqg_mpc_step a)
+{
+    constexpr int NX = P::NX, NU = P::NU, RXU = Rec<P>::RXU, KB = 8;
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= w.B) return;
+    const size_t Bp = w.Bp;
+    const int T = w.T, n = a.n_shift;
+    const double *src = w.XU[w.cur[b]];
+    const size_t row = (size_t)b * a.n_steps + a.step;
+    double xn[NX];
+#pragma unroll
+    for (int i = 0; i < NX; i++) {
+        xn[i] = src[((size_t)n * Bp + b) * RXU + i];
+        if (a.w) xn[i] = xn[i] + a.w[row * NX + i];
+    }
+    if (a.x_log) {
+        double *xl = a.x_log + ((size_t)b * (a.n_steps + 1) + a.step) * NX;
+#pragma unroll
+        for (int i = 0; i < NX; i++) xl[i] = w.x0[(size_t)i * Bp + b];
+        if (!a.plan)
+#pragma unroll
+            for (int i = 0; i < NX; i++) xl[NX + i] = xn[i];
+    }
+    if (a.u_log)
+#pragma unroll
+        for (int j = 0; j < NU; j++) a.u_log[row * NU + j] = src[(size_t)b * RXU + NX + j];
+    if (a.cost_log) a.cost_log[row] = w.cost[b];
+    if (a.it_log) a.it_log[row] = w.iterations[b];
+    if (a.res_log) a.res_log[row] = w.result[b];
+    if (!a.plan) return;
+    if (a.set_x0)
+#pragma unroll
+        for (int i = 0; i < NX; i++) w.x0[(size_t)i * Bp + b] = xn[i];
+    double *dst = w.XU[0];
+    for (int k0 = 0; k0 < T; k0 += KB) {
+        double u[KB][NU];
+#pragma unroll
+        for (int j = 0; j < KB; j++) {
+            const int ks = min(k0 + j + n, T - 1);   /* past the end: the last control, still unwritten (only step T-1 writes it) */
+            if (k0 + j < T)
+#pragma unroll
+                for (int i = 0; i < NU; i++) u[j][i] = src[((size_t)ks * Bp + b) * RXU + NX + i];
+        }
+#pragma unroll
+        for (int j = 0; j < KB; j++)
+            if (k0 + j < T)
+#pragma unroll
+                for (int i = 0; i < NU; i++) dst[((size_t)(k0 + j) * Bp + b) * RXU + NX + i] = u[j][i];
+    }
+}
+
 /* layout changes between the caller's problem-major arrays [B][n_k][n_i] and device arrays addressed as
  * base[(k * stride_k + b) * stride_b + off + i * stride_i]  (records: stride_k = Bp, stride_b = record size, stride_i = 1;
  * structure-of-arrays [k][i][Bp]: handled by the caller passing stride_b = 1, stride_i = Bp, stride_k = n_i * Bp / 1) */

@@ -52,4 +52,16 @@ typedef struct ilqg_work {
     int *tr_clamp;                  /* [T][Bp]: is_clamped of the last back pass, 2 bits per input, QP code << 16 */
 } ilqg_work;
 
+/* one receding-horizon step of every problem (k_mpc_advance).  The disturbance and the logs are problem-major
+ * ([B][n_steps][..], x_log [B][n_steps + 1][NX]) so that they copy to and from the caller's arrays without a layout change. */
+typedef struct ilqg_mpc_step {
+    int n_shift;        /* u[k] <- u[k + n_shift] for k < T - n_shift, u[T-1] after that */
+    int set_x0;         /* 1: x0 <- x[n_shift] (+ w); 0: x0 is left to the caller */
+    int plan;           /* 0: log only (the last step of a closed loop): the solution stays in place */
+    int step, n_steps;  /* row of w and of the logs */
+    const double *w;    /* [B][n_steps][NX] disturbance added to x[n_shift], or null */
+    double *x_log, *u_log, *cost_log;   /* x0 of the solve (and, log only, the next state), u[0], cost; null = not logged */
+    int *it_log, *res_log;              /* iterations, result */
+} ilqg_mpc_step;
+
 #endif

@@ -78,6 +78,8 @@ class Library:
         L.ilqgb_iterate.argtypes = [vp, ci]
         L.ilqgb_download.argtypes = [vp, dp, dp, dp, dp, dp, dp]
         L.ilqgb_solve_host.argtypes = [vp, dp, dp, dp, dp, dp, dp, dp, dp]
+        L.ilqgb_shift.argtypes = [vp, ci, dp, dp]
+        L.ilqgb_mpc.argtypes = [vp, ci, dp, dp, dp, dp, dp, dp, dp, dp]
         L.ilqgb_get.restype = C.c_long
         L.ilqgb_get.argtypes = [vp, cp, dp]
         L.ilqgb_get_int.restype = C.c_long
@@ -229,6 +231,39 @@ class BatchSolver:
         it = np.empty(self.B, np.int32); res = np.empty(self.B, np.int32); nls = np.empty(self.B, np.int32)
         self._chk(self.lib.ilqgb_solve_host(self.h, _ptr(x0), _ptr(u0), _ptr(x), _ptr(u), _ptr(cost), _ptr(it), _ptr(res), _ptr(nls)))
         return dict(success=res, x=x, u=u, cost=cost, iterations=it, n_linesearch=nls)
+
+    # receding horizon ----------------------------------------------------------------------------------------------------
+    def _state(self, name, a, shape):
+        if a is None:
+            return None
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        if a.shape != shape:
+            raise ValueError(f"wrong number of elements in {name} ({'x'.join(map(str, shape))} expected)")
+        return a
+
+    def shift(self, n=1, x0=None, w=None):
+        """The current solution becomes the next solve's input (ilqgb_shift): u[k] <- u[k+n], the last control repeated;
+        x0 <- x0 if given, else x[n] (+ w [B, nx]).  Needs a start since the last upload or shift."""
+        x0 = self._state("x0", x0, (self.B, self.nx))
+        w = self._state("w", w, (self.B, self.nx))
+        self._chk(self.lib.ilqgb_shift(self.h, int(n), _ptr(x0), _ptr(w)))
+        self._keep = (x0, w)
+
+    def mpc(self, x0, u0, n_steps, w=None):
+        """n_steps closed-loop steps on the device (ilqgb_mpc): solve, apply u[0], x0 <- x[1] + w[:, step], shift by one.
+        x0 = u0 = None continues from the current input (after upload or shift).  Returns the logs: x [B, S+1, nx] (the x0 of
+        every solve, then the final state), u [B, S, nu] (applied controls), cost, iterations, success [B, S].  The handle then
+        holds the last step's solution (download() returns the final plan)."""
+        S = int(n_steps)
+        if (x0 is None) != (u0 is None):
+            raise ValueError("x0 and u0 go together (neither: continue from the current input)")
+        x0 = self._state("x0", x0, (self.B, self.nx))
+        u0 = self._state("u_nom", u0, (self.B, self.T, self.nu))
+        w = self._state("w", w, (self.B, S, self.nx))
+        out = dict(x=np.empty((self.B, S + 1, self.nx)), u=np.empty((self.B, S, self.nu)), cost=np.empty((self.B, S)),
+                   iterations=np.empty((self.B, S), np.int32), success=np.empty((self.B, S), np.int32))
+        self._chk(self.lib.ilqgb_mpc(self.h, S, _ptr(x0), _ptr(u0), _ptr(w), *[_ptr(out[k]) for k in ("x", "u", "cost", "iterations", "success")]))
+        return out
 
     def set_tuning(self, name, value):
         """Run-time tuning knobs (ilqgb_set_tuning): ls_tail_from, bp_latency, bp_split, cw_lpp, pass_index."""

@@ -34,6 +34,14 @@ def normal(seed, stream, idx):
     return np.sqrt(-2.0 * np.log(u1)) * np.cos(2.0 * np.pi * u2)
 
 
+# ---- closed loops ------------------------------------------------------------------------------------------------------
+def disturbance(B, S, nx, scale, seed, first=0):
+    """Process noise of a closed loop, w [B, S, nx] = scale * N(0,1), for problems first..first+B-1 and steps 0..S-1."""
+    b = np.arange(first, first + B, dtype=np.uint64)
+    idx = np.arange(S * nx, dtype=np.uint64)[None, :]
+    return scale * normal(seed, b[:, None], idx).reshape(B, S, nx)
+
+
 # ---- car parking ---------------------------------------------------------------------------------------------
 CAR_PARAMS = {
     "d": [2.0], "h": [0.03],

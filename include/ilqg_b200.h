@@ -18,6 +18,8 @@
  *   ilqgb_finish                   iLQG.c:365-378 (iteration-limit bookkeeping)
  *   ilqgb_solve                    = start + iterate(max_iter) + finish: the whole iLQG() call for B problems
  *   ilqgb_download                 copy-out of x, u, cost, iLQG_mex.c:127-137, plus iterations / return value
+ *   ilqgb_shift / ilqgb_mpc        what a receding-horizon caller does between two iLQG_mex calls (SURVEY.md:211: the
+ *                                  previous u, shifted, is the next u_nom), on the device; ilqgb_mpc runs whole closed loops
  *   ilqgb_phase_*                  calc_derivs / back_pass / line_search on their own (iLQG.h:83, back_pass.h:7,
  *                                  line_search.h:6) for phase-level parity tests
  *   ilqgb_get / ilqgb_get_int      read-back of any per-problem field (tOptSet / trajEl_t members)
@@ -88,6 +90,22 @@ int ilqgb_sync(ilqgb_handle *h);
 int ilqgb_solve_host(ilqgb_handle *h, const double *x0, const double *u_nom, double *x, double *u, double *cost,
                      int *iterations, int *result, int *n_linesearch);
 int ilqgb_active(ilqgb_handle *h); /* problems still running (synchronises) */
+
+/* Receding horizon.  One closed-loop step is one reference call (upload + solve, every counter, lambda, penalty weight and
+ * multiplier re-initialised); [k]-indexed parameters are not shifted.  A problem whose solve failed (result 0 or -1) goes on
+ * with whatever its nominal trajectory holds, as a host loop over ilqgb_solve would.
+ * The current solution of every problem becomes the input of the next solve (the reference's caller does this by hand between
+ * two iLQG_mex calls): u[k] <- u[k+n_shift] (k < n_hor-n_shift), u[n_hor-1] after that; x0 <- x0 (host [batch][nx]) if given,
+ * else the solution's state x[n_shift] (+ w[batch][nx] if w != NULL; w requires x0 == NULL).  0 <= n_shift <= n_hor; requires
+ * ilqgb_start since the last upload / shift.  Asynchronous. */
+int ilqgb_shift(ilqgb_handle *h, int n_shift, const double *x0, const double *w);
+/* n_steps >= 1 closed-loop steps entirely on the device: solve, log, apply u[0], x0 <- x[1] + w[step], shift by one.
+ * x0 / u_nom: as ilqgb_upload, or both NULL = start from the handle's current input (last upload or shift).
+ * w [batch][n_steps][nx] or NULL.  Logs (any may be NULL): x_cl [batch][n_steps+1][nx], u_cl [batch][n_steps][nu],
+ * cost / iterations / result [batch][n_steps].  Afterwards the handle holds the LAST step's solution (not shifted), so
+ * ilqgb_download / ilqgb_get return the final plan.  Every chunk advances through the steps on its own.  Synchronises. */
+int ilqgb_mpc(ilqgb_handle *h, int n_steps, const double *x0, const double *u_nom, const double *w,
+              double *x_cl, double *u_cl, double *cost, int *iterations, int *result);
 
 /* device -> host; any pointer may be NULL. x [batch][n_hor+1][nx], u [batch][n_hor][nu] */
 int ilqgb_download(ilqgb_handle *h, double *x, double *u, double *cost, int *iterations, int *result,
