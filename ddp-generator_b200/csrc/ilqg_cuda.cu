@@ -67,14 +67,22 @@ template <class F> static int preload_one(F *f)
     cudaFuncAttributes a;
     return cudaFuncGetAttributes(&a, f) == cudaSuccess ? 0 : -1;
 }
-template <bool PP> static int preload_pp()
+/* the kernels that evaluate the problem functions, for shared [k]-indexed parameters or (TR) per-problem tracks */
+template <bool PP, bool TR> static int preload_pk()
 {
     constexpr bool FULL = FULL_DDP != 0;
     int bad = 0;
-    bad |= preload_one(k_init<P, PP>) | preload_one(k_rollout_only<P, PP>) | preload_one(k_derivs<P, FULL, PP>);
-    bad |= preload_one(k_ls_round<P, PP>) | preload_one(k_ls_tail<P, PP, true>) | preload_one(k_ls_tail<P, PP, false>);
-    bad |= preload_one(k_ls_commit_seg<P, PP>) | preload_one(k_ls_commit<P, PP, true>) | preload_one(k_ls_commit<P, PP, false>);
-    bad |= preload_one(k_post<P, PP>) | preload_one(k_mult<P, PP>) | preload_one(k_dense<P, PP>) | preload_one(k_clamp<P, PP>) | preload_one(k_eval<P, PP>);
+    bad |= preload_one(k_init<P, PP, TR>) | preload_one(k_rollout_only<P, PP, TR>) | preload_one(k_derivs<P, FULL, PP, TR>);
+    bad |= preload_one(k_ls_round<P, PP, TR>) | preload_one(k_ls_tail<P, PP, true, TR>) | preload_one(k_ls_tail<P, PP, false, TR>);
+    bad |= preload_one(k_ls_commit_seg<P, PP, TR>) | preload_one(k_ls_commit<P, PP, true, TR>) | preload_one(k_ls_commit<P, PP, false, TR>);
+    bad |= preload_one(k_post<P, PP, TR>) | preload_one(k_mult<P, PP, TR>) | preload_one(k_clamp<P, PP, TR>) | preload_one(k_eval<P, PP, TR>);
+    return bad;
+}
+template <bool PP> static int preload_pp()
+{
+    constexpr bool FULL = FULL_DDP != 0;
+    int bad = preload_pk<PP, false>() | preload_one(k_dense<P, PP>);
+    if constexpr (P::NKP > 0) bad |= preload_pk<PP, true>();   /* track variants exist only where there are [k]-indexed parameters */
     if constexpr (use_coop<P>()) {
         bad |= preload_one(k_backpass_warp<P, FULL, PP, 32>) | preload_one(k_backpass_warp<P, FULL, PP, 16>) | preload_one(k_backpass_warp<P, FULL, PP, 8>);
     } else {
@@ -166,23 +174,31 @@ static inline unsigned nblk(int n, int bs) { return (unsigned)((n + bs - 1) / bs
     do {                               \
         if ((w_)->pp) { constexpr bool PP = true; CALL; } else { constexpr bool PP = false; CALL; } \
     } while (0)
+/* the kernels that evaluate the problem functions also exist, for problems with [k]-indexed parameters, in a variant that
+   reads per-problem tracks (TR); without such parameters both branches name the same instantiation */
+constexpr bool HAS_KP = P::NKP > 0;
+#define PK_DISPATCH(w_, CALL)                                                                                         \
+    do {                                                                                                              \
+        if (HAS_KP && (w_)->tr_mask) { constexpr bool TR = HAS_KP; PP_DISPATCH(w_, CALL); }                            \
+        else { constexpr bool TR = false; PP_DISPATCH(w_, CALL); }                                                    \
+    } while (0)
 
 int ilqgk_launch_init(const ilqg_work *w, const ilqg_opts *o, const double *params, int mode, void *stream)
 {
-    PP_DISPATCH(w, (k_init<P, PP><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, make_pb(params), mode)));
+    PK_DISPATCH(w, (k_init<P, PP, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, make_pb(params), mode)));
     return check(cudaGetLastError(), "k_init");
 }
 
 int ilqgk_launch_rollout(const ilqg_work *w, const double *params, double alpha, int cost_only, void *stream)
 {
-    PP_DISPATCH(w, (k_rollout_only<P, PP><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, make_pb(params), alpha, cost_only)));
+    PK_DISPATCH(w, (k_rollout_only<P, PP, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, make_pb(params), alpha, cost_only)));
     return check(cudaGetLastError(), "k_rollout_only");
 }
 
 int ilqgk_launch_derivs(const ilqg_work *w, const double *params, void *stream)
 {
     dim3 grid(nblk(w->B, DV_BLOCK), (unsigned)(w->T + 1));
-    PP_DISPATCH(w, (k_derivs<P, FULL_DDP != 0, PP><<<grid, DV_BLOCK, 0, (cudaStream_t)stream>>>(*w, make_pb(params))));
+    PK_DISPATCH(w, (k_derivs<P, FULL_DDP != 0, PP, TR><<<grid, DV_BLOCK, 0, (cudaStream_t)stream>>>(*w, make_pb(params))));
     return check(cudaGetLastError(), "k_derivs");
 }
 
@@ -243,7 +259,7 @@ int ilqgk_launch_ls_reset(const ilqg_work *w, void *stream)
 
 int ilqgk_launch_ls_round(const ilqg_work *w, const ilqg_opts *o, const double *params, int iter, int round, void *stream)
 {
-    PP_DISPATCH(w, (k_ls_round<P, PP><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, make_pb(params), iter, round)));
+    PK_DISPATCH(w, (k_ls_round<P, PP, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, make_pb(params), iter, round)));
     return check(cudaGetLastError(), "k_ls_round");
 }
 
@@ -254,31 +270,31 @@ int ilqgk_launch_ls_tail(const ilqg_work *w, const ilqg_opts *o, const double *p
     const bool par = o->ls_commit_par && w->ls_ckpt;
     if (from == 0 && check(cudaMemsetAsync(w->ls_mask, 0, sizeof(int) * w->Bp, (cudaStream_t)stream), "memset ls_mask")) return -1;
     if (par)
-        PP_DISPATCH(w, (k_ls_tail<P, PP, true><<<nblk(w->B * nrem, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, from)));
+        PK_DISPATCH(w, (k_ls_tail<P, PP, true, TR><<<nblk(w->B * nrem, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, from)));
     else
-        PP_DISPATCH(w, (k_ls_tail<P, PP, false><<<nblk(w->B * nrem, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, from)));
+        PK_DISPATCH(w, (k_ls_tail<P, PP, false, TR><<<nblk(w->B * nrem, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, from)));
     if (check(cudaGetLastError(), "k_ls_tail")) return -1;
     if (par) {
         dim3 grid(nblk(w->B, BP_BLOCK), LS_SEGS);
-        PP_DISPATCH(w, (k_ls_commit_seg<P, PP><<<grid, BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, from)));
+        PK_DISPATCH(w, (k_ls_commit_seg<P, PP, TR><<<grid, BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, from)));
         if (check(cudaGetLastError(), "k_ls_commit_seg")) return -1;
-        PP_DISPATCH(w, (k_ls_commit<P, PP, true><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, iter, from)));
+        PK_DISPATCH(w, (k_ls_commit<P, PP, true, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, iter, from)));
     } else
-        PP_DISPATCH(w, (k_ls_commit<P, PP, false><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, iter, from)));
+        PK_DISPATCH(w, (k_ls_commit<P, PP, false, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, pb, iter, from)));
     return check(cudaGetLastError(), "k_ls_commit");
 }
 
 int ilqgk_launch_post(const ilqg_work *w, const ilqg_opts *o, const double *params, void *stream)
 {
     if (P::N_MU_R + P::N_MU_F == 0) return 0;   /* cost does not depend on multipliers/penalties: nothing to redo */
-    PP_DISPATCH(w, (k_post<P, PP><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, make_pb(params))));
+    PK_DISPATCH(w, (k_post<P, PP, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, make_pb(params))));
     return check(cudaGetLastError(), "k_post");
 }
 
 int ilqgk_launch_mult(const ilqg_work *w, const ilqg_opts *o, const double *params, int init, void *stream)
 {
     if (P::N_MU_R + P::N_MU_F == 0) return 0;
-    PP_DISPATCH(w, (k_mult<P, PP><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, make_pb(params), init)));
+    PK_DISPATCH(w, (k_mult<P, PP, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, *o, make_pb(params), init)));
     return check(cudaGetLastError(), "k_mult");
 }
 
@@ -293,7 +309,7 @@ int ilqgk_launch_dense(const ilqg_work *w, const double *params, double *out, vo
 
 int ilqgk_launch_clamp(const ilqg_work *w, const double *params, double *xu_io, int k, void *stream)
 {
-    PP_DISPATCH(w, (k_clamp<P, PP><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, make_pb(params), xu_io, k)));
+    PK_DISPATCH(w, (k_clamp<P, PP, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, make_pb(params), xu_io, k)));
     return check(cudaGetLastError(), "k_clamp");
 }
 
@@ -301,7 +317,7 @@ int ilqgk_eval_size(int mode) { return (mode >= 0 && mode <= 17) ? eval_size<P>(
 
 int ilqgk_launch_eval(const ilqg_work *w, const double *params, const double *in, double *out, int mode, int k, void *stream)
 {
-    PP_DISPATCH(w, (k_eval<P, PP><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, make_pb(params), in, out, mode, k)));
+    PK_DISPATCH(w, (k_eval<P, PP, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, make_pb(params), in, out, mode, k)));
     return check(cudaGetLastError(), "k_eval");
 }
 

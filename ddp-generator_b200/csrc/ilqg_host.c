@@ -35,7 +35,10 @@ struct chunk {
     ilqg_opts o;
     double *params;        /* flat, time-invariant */
     double *d_kp[16];      /* [k]-indexed parameters: device arrays of n_hor + 1 doubles, in parameter order */
-    double **d_pk;         /* device table of those pointers (ilqg_work.pk) */
+    double **d_pk;         /* device table of those pointers (ilqg_work.pk); a parameter with a track points to the track */
+    double *d_tr[16];      /* per-problem tracks [tr_len][Bp] of [k]-indexed parameters (ilqgb_set_param_track), or null;
+                              their window offset is w.tr_off and their bits are w.tr_mask */
+    int tr_len[16];
     double *d_pp;          /* per-problem parameter sets [npf][Bp] (ilqg_work.pp), allocated on first use */
     void *stream;          /* the stream all work of this chunk is enqueued on (stream_main, or stream_io during an end-to-end solve) */
     void *stream_main, *stream_io;
@@ -146,6 +149,7 @@ void ilqgb_mult_counts(int *n_running_eq, int *n_final_eq)
 int ilqgb_deriv_doubles_per_step(void) { ilqgk_dims_t d; ilqgk_dims(&d); return d.nv1 + (d.full_ddp ? d.nv2 : 0); }
 
 static void ck_destroy(chunk *h);
+static int ensure_stage(chunk *h, size_t doubles);
 
 /* ---- options (reference: standard_parameters iLQG.c:57-78, setOptParam iLQG.c:91-216) ----------------------------------- */
 static const double k_alpha_default[8] = {1.0, 0.3727594, 0.1389495, 0.0517947, 0.0193070, 0.0071969, 0.0026827, 0.0010000};
@@ -307,18 +311,65 @@ static int ck_set_param_batch(chunk *h, int index, const double *value, int n)
     return 0;
 }
 
+/* position of parameter `index` among the [k]-indexed ones */
+static int kp_index(int index)
+{
+    int i, kidx = 0;
+    for (i = 0; i < index; i++)
+        if (ilqgk_param_size(i) == -1) kidx++;
+    return kidx;
+}
+
+/* entry kidx of the device pointer table: the track if there is one, else the shared array */
+static int ck_point_pk(chunk *h, int kidx)
+{
+    const double *p = h->d_tr[kidx] ? h->d_tr[kidx] : h->d_kp[kidx];
+    if (ilqgk_h2d(h->d_pk + kidx, &p, sizeof p, h->stream) || ilqgk_stream_sync(h->stream)) return failk(h);
+    return 0;
+}
+
+static int ck_drop_track(chunk *h, int kidx)
+{
+    dfree(h, h->d_tr[kidx]);   /* cudaFree waits for the work that still reads it */
+    h->d_tr[kidx] = NULL;
+    h->tr_len[kidx] = 0;
+    h->w.tr_mask &= ~(1u << kidx);
+    return ck_point_pk(h, kidx);
+}
+
+/* the track of [k]-indexed parameter kidx for every problem of the chunk: value[b][len] (checked by the caller), moved to
+   [len][Bp] through the staging buffer by one layout kernel */
+static int ck_set_param_track(chunk *h, int kidx, const double *value, int len)
+{
+    const size_t n = (size_t)h->B * len;
+    if (ilqgk_set_device(h->device)) return failk(h);
+    if (h->d_tr[kidx] && h->tr_len[kidx] != len) {
+        dfree(h, h->d_tr[kidx]);
+        h->d_tr[kidx] = NULL;
+    }
+    if (!h->d_tr[kidx]) {
+        h->d_tr[kidx] = (double *)dalloc(h, sizeof(double) * (size_t)len * h->Bp);
+        if (!h->d_tr[kidx]) return -1;
+        h->tr_len[kidx] = len;
+    }
+    if (ensure_stage(h, n)) return -1;
+    if (ilqgk_h2d(h->d_stage, value, sizeof(double) * n, h->stream)) return failk(h);
+    if (ilqgk_launch_scatter(h->d_stage, h->d_tr[kidx], NULL, NULL, h->B, len, 1, h->Bp, 1, 0, 0, h->stream)) return failk(h);
+    h->n_launches++;
+    h->w.tr_mask |= 1u << kidx;
+    return ck_point_pk(h, kidx);
+}
+
 static int ck_set_param(chunk *h, int index, const double *value, int n)
 {
     int i, off = 0;
     if (index < 0 || index >= ilqgk_param_count()) return fail(h, "parameter index out of range");
     if (ilqgk_param_size(index) == -1) { /* one value per timestep, name[k] in the problem file */
-        int kidx = 0;
+        const int kidx = kp_index(index);
         if (n != h->T + 1) return fail(h, "wrong parameter length (n_hor + 1 expected)");
-        for (i = 0; i < index; i++)
-            if (ilqgk_param_size(i) == -1) kidx++;
         if (ilqgk_set_device(h->device)) return failk(h);
         if (ilqgk_h2d(h->d_kp[kidx], value, sizeof(double) * n, h->stream) || ilqgk_stream_sync(h->stream)) return failk(h);
-        return 0;
+        return h->d_tr[kidx] ? ck_drop_track(h, kidx) : 0;   /* shared and fixed again */
     }
     if (n != ilqgk_param_size(index)) return fail(h, "wrong parameter length");
     for (i = 0; i < index; i++)
@@ -649,7 +700,10 @@ static int ck_mpc_advance(chunk *h, int step)
     h->mpc.plan = step + 1 < h->mpc.n_steps;
     if (ilqgk_launch_mpc_advance(&h->w, &h->mpc, h->stream)) return failk(h);
     h->n_launches++;
-    if (h->mpc.plan) h->started = 0;   /* the input has been replaced */
+    if (h->mpc.plan) {
+        h->started = 0;   /* the input has been replaced */
+        h->w.tr_off++;    /* the tracks move with the plan: every later launch of this chunk passes the next window */
+    }
     return 0;
 }
 
@@ -1156,6 +1210,7 @@ struct ilqgb_handle {
     void *ev_fork, *ev_join[MAX_CHUNKS];
     int e2e_prio, e2e_stagger;   /* end-to-end solve: chunk streams with descending priority; start gate in passes */
     ilqgk_dims_t d;
+    int tr_off;        /* window offset of the parameter tracks (every chunk's w.tr_off between two calls) */
     char err[256];
 };
 
@@ -1336,6 +1391,59 @@ int ilqgb_set_param_batch(ilqgb_handle *h, int index, const double *value, int n
         if (ck_set_param_batch(h->c[i], index, value + (size_t)h->first[i] * n, n)) return hfail(h, h->c[i]);
     return 0;
 }
+
+/* ---- time-indexed parameter tracks (see ilqg_b200.h) ---- */
+/* length of the shortest track, 0 without tracks (every chunk holds the same tracks) */
+static int track_min_len(const ilqgb_handle *h)
+{
+    const chunk *c = h->c[0];
+    int j, m = 0;
+    for (j = 0; j < 16; j++)
+        if (c->d_tr[j] && (!m || c->tr_len[j] < m)) m = c->tr_len[j];
+    return m;
+}
+
+/* a window starting at `off` lies inside every track */
+static int window_fits(const ilqgb_handle *h, long long off)
+{
+    const int m = track_min_len(h);
+    return !m || off + h->T + 1 <= m;
+}
+
+static void set_track_offset(ilqgb_handle *h, int off)
+{
+    int i;
+    h->tr_off = off;
+    for (i = 0; i < h->n; i++) h->c[i]->w.tr_off = off;
+}
+
+int ilqgb_set_param_track(ilqgb_handle *h, int index, const double *value, int len)
+{
+    int i, kidx;
+    const int off = track_min_len(h) ? h->tr_off : 0;
+    if (index < 0 || index >= ilqgk_param_count()) { snprintf(h->err, sizeof h->err, "parameter index out of range"); return -1; }
+    if (ilqgk_param_size(index) != -1) { snprintf(h->err, sizeof h->err, "only [k]-indexed parameters have tracks"); return -1; }
+    if (!value) { snprintf(h->err, sizeof h->err, "no track values"); return -1; }
+    if ((long long)len < (long long)off + h->T + 1) {
+        snprintf(h->err, sizeof h->err, "track too short: len >= offset + n_hor + 1 = %lld expected", (long long)off + h->T + 1);
+        return -1;
+    }
+    kidx = kp_index(index);
+    set_track_offset(h, off);
+    for (i = 0; i < h->n; i++)
+        if (ck_set_param_track(h->c[i], kidx, value + (size_t)h->first[i] * len, len)) return hfail(h, h->c[i]);
+    return 0;
+}
+
+int ilqgb_set_track_offset(ilqgb_handle *h, int offset)
+{
+    if (offset < 0) { snprintf(h->err, sizeof h->err, "the track offset must be >= 0"); return -1; }
+    if (!window_fits(h, offset)) { snprintf(h->err, sizeof h->err, "offset + n_hor + 1 exceeds the length of a track"); return -1; }
+    set_track_offset(h, offset);
+    return 0;
+}
+
+int ilqgb_track_offset(const ilqgb_handle *h) { return h->tr_off; }
 
 int ilqgb_upload(ilqgb_handle *h, const double *x0, const double *u_nom)
 {
@@ -1568,11 +1676,16 @@ int ilqgb_shift(ilqgb_handle *h, int n_shift, const double *x0, const double *w)
     if (x0 && w) { snprintf(h->err, sizeof h->err, "w is added to the solution's state: it cannot go with x0"); return -1; }
     for (i = 0; i < h->n; i++)
         if (!h->c[i]->started) { snprintf(h->err, sizeof h->err, "ilqgb_start has not been called since the last upload or shift"); return -1; }
+    if (!window_fits(h, (long long)h->tr_off + n_shift)) {
+        snprintf(h->err, sizeof h->err, "offset + n_shift + n_hor + 1 exceeds the length of a track");
+        return -1;
+    }
     if (fork_streams(h)) return -1;
     for (i = 0; i < h->n; i++) {
         const size_t f = (size_t)h->first[i] * h->d.nx;
         if (ck_shift(h->c[i], n_shift, x0 ? x0 + f : NULL, w ? w + f : NULL)) return hfail(h, h->c[i]);
     }
+    set_track_offset(h, h->tr_off + n_shift);
     return join_streams(h);
 }
 
@@ -1583,14 +1696,21 @@ int ilqgb_mpc(ilqgb_handle *h, int n_steps, const double *x0, const double *u_no
               double *cost, int *iterations, int *result)
 {
     const mpc_t m = {n_steps, w, x_cl, u_cl, cost, iterations, result};
-    int i;
+    int i, rc;
     if (n_steps < 1) { snprintf(h->err, sizeof h->err, "n_steps must be >= 1"); return -1; }
     if (!x0 != !u_nom) { snprintf(h->err, sizeof h->err, "x0 and u_nom go together (neither: continue from the current input)"); return -1; }
     if (!x0)
         for (i = 0; i < h->n; i++)
             if (h->c[i]->started) { snprintf(h->err, sizeof h->err, "no input to continue from: ilqgb_upload or ilqgb_shift since the last start"); return -1; }
+    if (!window_fits(h, (long long)h->tr_off + n_steps - 1)) {
+        snprintf(h->err, sizeof h->err, "offset + (n_steps - 1) + n_hor + 1 exceeds the length of a track");
+        return -1;
+    }
     if (x0 && ilqgb_upload(h, x0, u_nom)) return -1;
-    if (run_engine(h, NULL, &m)) return -1;
+    /* each chunk moves its own offset as it shifts (ck_mpc_advance); all of them end n_steps - 1 further */
+    rc = run_engine(h, NULL, &m);
+    set_track_offset(h, rc ? h->tr_off : h->tr_off + n_steps - 1);
+    if (rc) return -1;
     return ilqgb_sync(h);
 }
 

@@ -58,6 +58,35 @@ template <class P> struct ParamBlock { double v[P::NPF]; };
         pv = pl_;                                                                              \
     }
 
+/* [k]-indexed parameters (name[k] in a problem file), read by the generated problem functions as pk(j, k).  PkShared: one
+   array of n_hor + 1 values per parameter, shared by the batch (w.pk[j][k]).  PkTrack (ilqgb_set_param_track): the parameters
+   whose bit is set in w.tr_mask have a track per problem, stored [len][Bp] with the problem index fastest so that the lanes of
+   a warp read one coalesced row, and a solve reads step w.tr_off + k of it; the others stay shared.  The bit test is uniform
+   over a launch.  Only the kernels that evaluate the problem functions have a track variant (template flag TR); the
+   backward passes read derivative entries and consts(p) alone. */
+struct PkShared {
+    const double *const *p;
+    __device__ __forceinline__ double operator()(int j, int k) const { return p[j][k]; }
+};
+struct PkTrack {
+    const double *const *p;
+    unsigned mask;
+    int off, b;
+    size_t Bp;
+    __device__ __forceinline__ double operator()(int j, int k) const
+    {
+        return ((mask >> j) & 1u) ? p[j][(size_t)(off + k) * Bp + b] : p[j][k];
+    }
+};
+template <bool TR> struct PkSel { using type = PkShared; };
+template <> struct PkSel<true> { using type = PkTrack; };
+template <bool TR> __device__ __forceinline__ typename PkSel<TR>::type make_pk(const ilqg_work &w, int b)
+{
+    if constexpr (TR) return PkTrack{w.pk, w.tr_mask, w.tr_off, b, (size_t)w.Bp};
+    else return PkShared{w.pk};
+}
+#define ILQG_PK(TR_, b_) const auto pk = make_pk<TR_>(w, (b_));
+
 #ifndef ILQG_FORCE_COOP
 #define ILQG_FORCE_COOP 0
 #endif
@@ -446,7 +475,7 @@ __device__ __forceinline__ void rewrite8(double *p)
     *p = v;
 }
 
-template <class P, bool FULL, bool PP>
+template <class P, bool FULL, bool PP, bool TR = false>
 __global__ void __launch_bounds__(DV_BLOCK) k_derivs(Work w, ParamBlock<P> pb)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -486,6 +515,7 @@ __global__ void __launch_bounds__(DV_BLOCK) k_derivs(Work w, ParamBlock<P> pb)
         return;
     }
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     const int cur = w.cur[b];
     constexpr int RXU = Rec<P>::RXU;
     double xu[RXU], mu[P::N_MU_R + P::N_MU_F + 1];
@@ -498,9 +528,9 @@ __global__ void __launch_bounds__(DV_BLOCK) k_derivs(Work w, ParamBlock<P> pb)
         double v1[P::NV1], v2[P::NV2];
         const double w_pen = w.w_pen_l[b];
         if (FULL)
-            ok = P::derivs_full(x, u, pv, w.pk, k, w.T, w_pen, mu, v1, v2);
+            ok = P::derivs_full(x, u, pv, pk, k, w.T, w_pen, mu, v1, v2);
         else
-            ok = P::derivs(x, u, pv, w.pk, k, w.T, w_pen, mu, v1, v2);
+            ok = P::derivs(x, u, pv, pk, k, w.T, w_pen, mu, v1, v2);
         if (use_coop<P>()) { /* one contiguous record per (step, problem): the consumer is a whole warp per problem */
             double *o1 = w.V1 + ((size_t)k * Bp + b) * P::NV1;
 #pragma unroll
@@ -524,7 +554,7 @@ __global__ void __launch_bounds__(DV_BLOCK) k_derivs(Work w, ParamBlock<P> pb)
 #pragma unroll
         for (int i = 0; i < P::N_MU_F; i++) mu[i] = w.muF[(size_t)i * Bp + b];
         double cx[P::NX], cxx[P::NQXX];
-        ok = P::derivs_final(x, pv, w.pk, w.T, w.T, w.w_pen_f[b], mu, cx, cxx);
+        ok = P::derivs_final(x, pv, pk, w.T, w.T, w.w_pen_f[b], mu, cx, cxx);
         double *fd = w.FD + b;
 #pragma unroll
         for (int i = 0; i < P::NX; i++) fd[i * Bp] = cx[i];
@@ -1340,8 +1370,8 @@ namespace ilqg {
 constexpr int LS_SEGS = 32;
 __host__ __device__ inline int ls_seg_len(int T) { return (T + LS_SEGS - 1) / LS_SEGS; }
 
-template <class P, bool STORE = true, bool CKPT = false>
-__device__ __forceinline__ bool rollout(const Work &w, const double *pv, int b, int from, int to, double alpha,
+template <class P, bool STORE = true, bool CKPT = false, class PK>
+__device__ __forceinline__ bool rollout(const Work &w, const double *pv, const PK &pk, int b, int from, int to, double alpha,
                                         double w_pen_l, double w_pen_f, double &csum, double *ckpt = nullptr)
 {
     constexpr int NX = P::NX, NU = P::NU, RXU = Rec<P>::RXU, RLM = Rec<P>::RLM, RLS = Rec<P>::RLS, RLL = NU + RLM;
@@ -1405,7 +1435,7 @@ __device__ __forceinline__ bool rollout(const Work &w, const double *pv, int b, 
 #pragma unroll
         for (int i = 0; i < P::N_MU_R; i++) mu[i] = w.muR[((size_t)k * P::N_MU_R + i) * Bp + b];
         double c;
-        const bool ok = P::step(x, u, pv, w.pk, k, T, w_pen_l, mu, xn, c);
+        const bool ok = P::step(x, u, pv, pk, k, T, w_pen_l, mu, xn, c);
         if (STORE) st_rec<RXU>(w.XU[to] + ((size_t)k * Bp + b) * RXU, xu);
         if (!ok) return false;
         csum += c;
@@ -1424,14 +1454,14 @@ __device__ __forceinline__ bool rollout(const Work &w, const double *pv, int b, 
 #pragma unroll
     for (int i = 0; i < P::N_MU_F; i++) mu[i] = w.muF[(size_t)i * Bp + b];
     double c;
-    if (!P::final_cost(x, pv, w.pk, T, T, w_pen_f, mu, c)) return false;
+    if (!P::final_cost(x, pv, pk, T, T, w_pen_f, mu, c)) return false;
     csum += c;
     return true;
 }
 
 /* cost-only pass over the nominal trajectory (forward_pass with cost_only = 1) */
-template <class P>
-__device__ __forceinline__ bool cost_pass(const Work &w, const double *pv, int b, int buf, double w_pen_l,
+template <class P, class PK>
+__device__ __forceinline__ bool cost_pass(const Work &w, const double *pv, const PK &pk, int b, int buf, double w_pen_l,
                                           double w_pen_f, double &csum)
 {
     constexpr int NX = P::NX, NU = P::NU, RXU = Rec<P>::RXU;
@@ -1444,14 +1474,14 @@ __device__ __forceinline__ bool cost_pass(const Work &w, const double *pv, int b
 #pragma unroll
         for (int i = 0; i < P::N_MU_R; i++) mu[i] = w.muR[((size_t)k * P::N_MU_R + i) * Bp + b];
         double c;
-        if (!P::step_cost(xu, xu + NX, pv, w.pk, k, T, w_pen_l, mu, c)) return false;
+        if (!P::step_cost(xu, xu + NX, pv, pk, k, T, w_pen_l, mu, c)) return false;
         csum += c;
     }
     ld_rec<NX>(w.XU[buf] + ((size_t)T * Bp + b) * RXU, xu);
 #pragma unroll
     for (int i = 0; i < P::N_MU_F; i++) mu[i] = w.muF[(size_t)i * Bp + b];
     double c;
-    if (!P::final_cost(xu, pv, w.pk, T, T, w_pen_f, mu, c)) return false;
+    if (!P::final_cost(xu, pv, pk, T, T, w_pen_f, mu, c)) return false;
     csum += c;
     return true;
 }
@@ -1460,8 +1490,8 @@ __device__ __forceinline__ bool cost_pass(const Work &w, const double *pv, int b
 /* Steps [k0, k1) of a rollout whose state at step k0 is known (recorded by a checkpointing rollout): the same operations
  * in the same order as rollout(), hence the same bits, always with stores.  The segment that ends at T also writes the
  * final record. */
-template <class P>
-__device__ __forceinline__ void rollout_segment(const Work &w, const double *pv, int b, int from, int to, double alpha,
+template <class P, class PK>
+__device__ __forceinline__ void rollout_segment(const Work &w, const double *pv, const PK &pk, int b, int from, int to, double alpha,
                                                 double w_pen_l, int k0, int k1, const double *xs)
 {
     constexpr int NX = P::NX, NU = P::NU, RXU = Rec<P>::RXU, RLM = Rec<P>::RLM, RLS = Rec<P>::RLS, RLL = NU + RLM;
@@ -1493,7 +1523,7 @@ __device__ __forceinline__ void rollout_segment(const Work &w, const double *pv,
 #pragma unroll
         for (int i = 0; i < P::N_MU_R; i++) mu[i] = w.muR[((size_t)k * P::N_MU_R + i) * Bp + b];
         double c;
-        P::step(x, u, pv, w.pk, k, T, w_pen_l, mu, xn, c);
+        P::step(x, u, pv, pk, k, T, w_pen_l, mu, xn, c);
         st_rec<RXU>(w.XU[to] + ((size_t)k * Bp + b) * RXU, xu);
 #pragma unroll
         for (int i = 0; i < NX; i++) x[i] = xn[i];
@@ -1509,8 +1539,8 @@ __device__ __forceinline__ void rollout_segment(const Work &w, const double *pv,
  * the constraint values: of step 0 for the running constraints -- the reference's early return sits INSIDE the loop over the
  * steps (iLQG_func.tem:452) -- and of the final ones; it never touches multipliers or penalty weights.  The multiplier
  * updates use the penalty weights the call started with, like the reference's local copies. */
-template <class P>
-__device__ __forceinline__ void update_mult(const Work &w, const Opts &o, const double *pv, int b, int buf, bool init,
+template <class P, class PK>
+__device__ __forceinline__ void update_mult(const Work &w, const Opts &o, const double *pv, const PK &pk, int b, int buf, bool init,
                                             double &w_pen_l, double &w_pen_f)
 {
     constexpr int NX = P::NX, NU = P::NU, NR = P::N_MU_R, NF = P::N_MU_F;
@@ -1529,7 +1559,7 @@ __device__ __forceinline__ void update_mult(const Work &w, const Opts &o, const 
             for (int j = 0; j < NU; j++) u[j] = xu[NX + j];
 #pragma unroll
             for (int i = 0; i < NR; i++) mu[i] = w.muR[((size_t)k * NR + i) * Bp + b];
-            P::mult_running(x, u, pv, w.pk, k, T, w_pen_l, mu, hval, mun);
+            P::mult_running(x, u, pv, pk, k, T, w_pen_l, mu, hval, mun);
 #pragma unroll
             for (int i = 0; i < NR; i++) {
                 double *last = &w.lastR[((size_t)k * NR + i) * Bp + b];
@@ -1549,7 +1579,7 @@ __device__ __forceinline__ void update_mult(const Work &w, const Opts &o, const 
         ld_rec<NX>(w.XU[buf] + ((size_t)T * Bp + b) * Rec<P>::RXU, x);
 #pragma unroll
         for (int i = 0; i < NF; i++) mu[i] = w.muF[(size_t)i * Bp + b];
-        P::mult_final(x, pv, w.pk, T, T, w_pen_f, mu, hval, mun);
+        P::mult_final(x, pv, pk, T, T, w_pen_f, mu, hval, mun);
 #pragma unroll
         for (int i = 0; i < NF; i++) {
             double *last = &w.lastF[(size_t)i * Bp + b];
@@ -1567,12 +1597,13 @@ __device__ __forceinline__ void update_mult(const Work &w, const Opts &o, const 
 
 enum { INIT_MULT = 1, INIT_ROLLOUT = 2, INIT_BEGIN = 4, INIT_ALL = 7 };
 
-template <class P, bool PP>
+template <class P, bool PP, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK) k_init(Work w, Opts o, ParamBlock<P> pb, int mode)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= w.B) return;
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     const size_t Bp = w.Bp;
     const int T = w.T;
     if (mode & INIT_MULT) { /* init_multipliers (iLQG_func.tem:364-400) */
@@ -1594,7 +1625,7 @@ __global__ void __launch_bounds__(BP_BLOCK) k_init(Work w, Opts o, ParamBlock<P>
     bool ok = true;
     if (mode & INIT_ROLLOUT) {
         double csum;
-        ok = rollout<P>(w, pv, b, 0, 1, 0.0, 0.0, 0.0, csum);
+        ok = rollout<P>(w, pv, pk, b, 0, 1, 0.0, 0.0, 0.0, csum);
         w.cur[b] = 1;
         w.cost[b] = csum;
         w.new_cost[b] = csum;
@@ -1625,23 +1656,24 @@ __global__ void __launch_bounds__(BP_BLOCK) k_init(Work w, Opts o, ParamBlock<P>
     w.new_deriv[b] = 1;
     if (ok && (P::N_MU_R + P::N_MU_F) > 0) { /* update_multipliers(o, 1), iLQG.c:236 */
         double wl = o.w_pen_init_l, wf = o.w_pen_init_f;
-        update_mult<P>(w, o, pv, b, nb, true, wl, wf);
+        update_mult<P>(w, o, pv, pk, b, nb, true, wl, wf);
     }
 }
 
 /* forward_pass(candidate, o, alpha, &csum, cost_only) of the single-problem API on its own (iLQG_func.tem:121-185):
  * one rollout from the nominal buffer into the other one (or the cost-only pass over the nominal); csum -> new_cost,
  * success flag -> result.  No solver bookkeeping. */
-template <class P, bool PP>
+template <class P, bool PP, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK) k_rollout_only(Work w, ParamBlock<P> pb, double alpha, int cost_only)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= w.B) return;
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     const int cur = w.cur[b];
     double csum;
-    const bool ok = cost_only ? cost_pass<P>(w, pv, b, cur, w.w_pen_l[b], w.w_pen_f[b], csum)
-                              : rollout<P>(w, pv, b, cur, cur ^ 1, alpha, w.w_pen_l[b], w.w_pen_f[b], csum);
+    const bool ok = cost_only ? cost_pass<P>(w, pv, pk, b, cur, w.w_pen_l[b], w.w_pen_f[b], csum)
+                              : rollout<P>(w, pv, pk, b, cur, cur ^ 1, alpha, w.w_pen_l[b], w.w_pen_f[b], csum);
     w.new_cost[b] = csum;
     w.result[b] = ok ? 1 : 0;
 }
@@ -1686,7 +1718,7 @@ __device__ __forceinline__ void ls_decide(const Work &w, const Opts &o, int b, i
  * while one neighbour backtracks.  The list keeps the problems of a block in order, which keeps most 32-byte
  * sectors shared between neighbouring lanes.  The problem that accepts, or exhausts the alphas, runs the
  * accept/reject bookkeeping of iLQG.c:311-361 in the same thread. */
-template <class P, bool PP>
+template <class P, bool PP, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS)
 k_ls_round(Work w, Opts o, ParamBlock<P> pb, int iter, int round)
 {
@@ -1701,6 +1733,7 @@ k_ls_round(Work w, Opts o, ParamBlock<P> pb, int iter, int round)
     bool undecided = false;
     if (b >= 0) {
         ILQG_PARAMS(PP, b)
+        ILQG_PK(TR, b)
         const int cur = w.cur[b];
         const double cost = w.cost[b], dV0 = w.dV0[b], dV1 = w.dV1[b];
         double w_pen_l = w.w_pen_l[b], w_pen_f = w.w_pen_f[b];
@@ -1712,7 +1745,7 @@ k_ls_round(Work w, Opts o, ParamBlock<P> pb, int iter, int round)
         w.n_roll[b] += 1;
         const double alpha = o.alpha[round];
         bool accepted = false;
-        const bool ok = rollout<P>(w, pv, b, cur, cur ^ 1, alpha, w_pen_l, w_pen_f, cnew);
+        const bool ok = rollout<P>(w, pv, pk, b, cur, cur ^ 1, alpha, w_pen_l, w_pen_f, cnew);
         if (ok) {
             dcost = cost - cnew;
             expected = -alpha * (dV0 + alpha * dV1);
@@ -1758,7 +1791,7 @@ k_ls_round(Work w, Opts o, ParamBlock<P> pb, int iter, int round)
  * (problem, alpha), without storing trajectories; k_ls_commit then replays the reference's sequential decision over
  * the recorded costs (first alpha with z > zMin wins, line_search.c:37-60) and re-runs only the winning rollout with
  * stores.  The line search then costs from + 2 rollout latencies instead of n_alpha; results are bit-identical. */
-template <class P, bool PP, bool CKPT>
+template <class P, bool PP, bool CKPT, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_ls_tail(Work w, Opts o, ParamBlock<P> pb, int from)
 {
     const int nrem = o.n_alpha - from;
@@ -1773,10 +1806,11 @@ __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_ls_tail(Work w,
         b = w.ls_list[from & 1][i];
     }
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     const int cur = w.cur[b];
     const double alpha = o.alpha[a];
     double cnew;
-    const bool ok = rollout<P, false, CKPT>(w, pv, b, cur, cur ^ 1, alpha, w.w_pen_l[b], w.w_pen_f[b], cnew,
+    const bool ok = rollout<P, false, CKPT>(w, pv, pk, b, cur, cur ^ 1, alpha, w.w_pen_l[b], w.w_pen_f[b], cnew,
                                             CKPT ? w.ls_ckpt + (size_t)a * LS_SEGS * w.Bp * P::NX : nullptr);
     w.ls_cnew[(size_t)a * w.Bp + b] = cnew;
     if (ok) {
@@ -1787,7 +1821,7 @@ __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_ls_tail(Work w,
     }
 }
 
-template <class P, bool PP, bool NOROLL>
+template <class P, bool PP, bool NOROLL, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_ls_commit(Work w, Opts o, ParamBlock<P> pb, int iter, int from)
 {
     const int tid = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1803,6 +1837,7 @@ __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_ls_commit(Work 
         b = w.ls_list[from & 1][tid];
     }
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     const int cur = w.cur[b];
     const int mask = w.ls_mask[b];
     const double cost = w.cost[b], dV0 = w.dV0[b], dV1 = w.dV1[b];
@@ -1826,7 +1861,7 @@ __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_ls_commit(Work 
     w.n_roll[b] += (win >= 0 ? 1 : 0);
     if (win >= 0 && !NOROLL) { /* NOROLL: k_ls_commit_seg has stored the winner's trajectory, its cost is the recorded one */
         double c2;
-        rollout<P, true>(w, pv, b, cur, cur ^ 1, o.alpha[win], w_pen_l, w_pen_f, c2); /* same arithmetic -> same cost */
+        rollout<P, true>(w, pv, pk, b, cur, cur ^ 1, o.alpha[win], w_pen_l, w_pen_f, c2); /* same arithmetic -> same cost */
         cnew = c2;
     }
     w.new_cost[b] = cnew;
@@ -1843,7 +1878,7 @@ __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_ls_commit(Work 
  * Every step repeats the tail's arithmetic on the same inputs, so the stored trajectory is bit-identical to the one the
  * sequential commit writes; k_ls_commit<.., NOROLL = true> follows with the bookkeeping and takes the cost from the tail's
  * record.  This kernel only reads solver state. */
-template <class P, bool PP>
+template <class P, bool PP, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_ls_commit_seg(Work w, Opts o, ParamBlock<P> pb, int from)
 {
     const int tid = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1863,17 +1898,18 @@ __global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_ls_commit_seg(W
     const int k0 = seg * seg_len, k1 = (k0 + seg_len < T) ? k0 + seg_len : T;
     if (k0 >= T) return;
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     const int cur = w.cur[b];
     double xs[P::NX];
     const double *c = w.ls_ckpt + (((size_t)win * LS_SEGS + seg) * w.Bp + b) * P::NX;
 #pragma unroll
     for (int i = 0; i < P::NX; i++) xs[i] = c[i];
-    rollout_segment<P>(w, pv, b, cur, cur ^ 1, o.alpha[win], w.w_pen_l[b], k0, k1, xs);
+    rollout_segment<P>(w, pv, pk, b, cur, cur ^ 1, o.alpha[win], w.w_pen_l[b], k0, k1, xs);
 }
 
 /* K5: update_multipliers(o, 0) and the cost-only pass that follows an accepted step, or the cost-only pass after a
  * rejected step whose penalty weights grew (iLQG.c:337-338, 345-349).  Only launched for problems with multipliers. */
-template <class P, bool PP>
+template <class P, bool PP, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK) k_post(Work w, Opts o, ParamBlock<P> pb)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1882,28 +1918,30 @@ __global__ void __launch_bounds__(BP_BLOCK) k_post(Work w, Opts o, ParamBlock<P>
     if (mode == POST_NONE) return;
     w.post_mode[b] = POST_NONE;
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     const int cur = w.cur[b];
     double w_pen_l = w.w_pen_l[b], w_pen_f = w.w_pen_f[b];
     if (mode == POST_MULT) {
-        update_mult<P>(w, o, pv, b, cur, false, w_pen_l, w_pen_f);
+        update_mult<P>(w, o, pv, pk, b, cur, false, w_pen_l, w_pen_f);
         w.w_pen_l[b] = w_pen_l;
         w.w_pen_f[b] = w_pen_f;
     }
     double csum;
-    cost_pass<P>(w, pv, b, cur, w_pen_l, w_pen_f, csum);
+    cost_pass<P>(w, pv, pk, b, cur, w_pen_l, w_pen_f, csum);
     w.cost[b] = csum;
 }
 
 
 /* update_multipliers(o, init) on its own (iLQG.h:86), for every running problem: the single-problem drop-in's entry point */
-template <class P, bool PP>
+template <class P, bool PP, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK) k_mult(Work w, Opts o, ParamBlock<P> pb, int init)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= w.B || w.status[b] != ST_RUNNING) return;
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     double w_pen_l = w.w_pen_l[b], w_pen_f = w.w_pen_f[b];
-    update_mult<P>(w, o, pv, b, w.cur[b], init != 0, w_pen_l, w_pen_f);
+    update_mult<P>(w, o, pv, pk, b, w.cur[b], init != 0, w_pen_l, w_pen_f);
     w.w_pen_l[b] = w_pen_l;
     w.w_pen_f[b] = w_pen_f;
 }
@@ -1950,12 +1988,13 @@ __global__ void __launch_bounds__(DV_BLOCK) k_dense(Work w, ParamBlock<P> pb, do
 }
 
 /* clampU(u, t, k, p, N) (iLQG_func.tem:68-73) for a batch: xu[b] = x | u, the clamped u is written back in place */
-template <class P, bool PP>
+template <class P, bool PP, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK) k_clamp(Work w, ParamBlock<P> pb, double *xu_io, int k)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= w.B) return;
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     double x[P::NX], u[P::NU], xn[P::NX], mu[P::N_MU_R + P::N_MU_F + 1], c;
     double *io = xu_io + (size_t)b * (P::NX + P::NU);
 #pragma unroll
@@ -1964,7 +2003,7 @@ __global__ void __launch_bounds__(BP_BLOCK) k_clamp(Work w, ParamBlock<P> pb, do
     for (int i = 0; i < P::NU; i++) u[i] = io[P::NX + i];
 #pragma unroll
     for (int i = 0; i < P::N_MU_R; i++) mu[i] = 0.0;
-    P::step(x, u, pv, w.pk, k, w.T, 0.0, mu, xn, c);   /* the clamp is the first thing a step does to u */
+    P::step(x, u, pv, pk, k, w.T, 0.0, mu, xn, c);   /* the clamp is the first thing a step does to u */
 #pragma unroll
     for (int i = 0; i < P::NU; i++) io[P::NX + i] = u[i];
 }
@@ -1981,13 +2020,14 @@ template <class P> __host__ __device__ constexpr int eval_size(int mode)
          : mode == 13 ? P::NU * P::NU * P::NX : mode == 14 ? P::NX * P::NU * P::NX : mode == 16 ? P::NU : mode == 17 ? P::NG : 0;
 }
 
-template <class P, bool PP>
+template <class P, bool PP, bool TR = false>
 __global__ void __launch_bounds__(BP_BLOCK) k_eval(Work w, ParamBlock<P> pb, const double *in, double *out, int mode, int k)
 {
     constexpr int NX = P::NX, NU = P::NU, NQXX = P::NQXX, NQUU = P::NQUU, NQXU = P::NQXU;
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= w.B) return;
     ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
     double x[NX], u[NU], mu[P::N_MU_R + P::N_MU_F + 1];
 #pragma unroll
     for (int i = 0; i < NX; i++) x[i] = in[(size_t)b * (NX + NU) + i];
@@ -1999,7 +2039,7 @@ __global__ void __launch_bounds__(BP_BLOCK) k_eval(Work w, ParamBlock<P> pb, con
     const int T = w.T;
     if (mode == 0 || mode == 1) {
         double xn[NX], c;
-        P::step_free(x, u, pv, w.pk, k, T, 1.0, mu, xn, c);
+        P::step_free(x, u, pv, pk, k, T, 1.0, mu, xn, c);
         if (mode == 0) {
 #pragma unroll
             for (int i = 0; i < NX; i++) o_[i] = xn[i];
@@ -2007,11 +2047,11 @@ __global__ void __launch_bounds__(BP_BLOCK) k_eval(Work w, ParamBlock<P> pb, con
             o_[0] = c;
     } else if (mode == 2) {
         double c;
-        P::final_cost(x, pv, w.pk, T, T, 1.0, mu, c);
+        P::final_cost(x, pv, pk, T, T, 1.0, mu, c);
         o_[0] = c;
     } else if (mode == 3 || mode == 4) {
         double cx[NX], cxx[NQXX];
-        P::derivs_final(x, pv, w.pk, T, T, 1.0, mu, cx, cxx);
+        P::derivs_final(x, pv, pk, T, T, 1.0, mu, cx, cxx);
         if (mode == 3) {
 #pragma unroll
             for (int i = 0; i < NX; i++) o_[i] = cx[i];
@@ -2020,12 +2060,12 @@ __global__ void __launch_bounds__(BP_BLOCK) k_eval(Work w, ParamBlock<P> pb, con
                 for (int r = 0; r < NX; r++) o_[r + c * NX] = cxx[symtri(r, c)];
     } else if (mode == 17) {
         double g[P::NG + 1];
-        P::calc_g(x, u, pv, w.pk, k, T, 1.0, mu, g);
+        P::calc_g(x, u, pv, pk, k, T, 1.0, mu, g);
 #pragma unroll
         for (int i = 0; i < P::NG; i++) o_[i] = g[i];
     } else if (mode == 16) {
         double xn[NX], c;
-        P::step(x, u, pv, w.pk, k, T, 1.0, mu, xn, c);
+        P::step(x, u, pv, pk, k, T, 1.0, mu, xn, c);
 #pragma unroll
         for (int i = 0; i < NU; i++) o_[i] = u[i];
     } else if (mode >= 5 && mode <= 14) {
@@ -2034,7 +2074,7 @@ __global__ void __launch_bounds__(BP_BLOCK) k_eval(Work w, ParamBlock<P> pb, con
         for (int i = 0; i < P::DENSE_SIZE; i++) Dd[i] = 0.0;
         double v1[P::NV1], v2[P::NV2];
         P::consts(pv, D);
-        P::derivs_full(x, u, pv, w.pk, k, T, 1.0, mu, v1, v2);
+        P::derivs_full(x, u, pv, pk, k, T, 1.0, mu, v1, v2);
         P::unpack(v1, D);
         if (mode == 5) for (int i = 0; i < NX; i++) o_[i] = D.cx[i];
         if (mode == 6) for (int i = 0; i < NU; i++) o_[i] = D.cu[i];

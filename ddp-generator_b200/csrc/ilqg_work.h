@@ -50,6 +50,9 @@ typedef struct ilqg_work {
     double *tr_lambda, *tr_newcost, *tr_z; /* [max_iter][Bp]: lambda at the line search, last rollout cost, last z */
     int *tr_alpha;                  /* [max_iter][Bp] */
     int *tr_clamp;                  /* [T][Bp]: is_clamped of the last back pass, 2 bits per input, QP code << 16 */
+    /* time-indexed parameter tracks (appended: the kernel-argument offsets of the fields above do not move) */
+    unsigned tr_mask;               /* bit j: pk[j] is a track [len][Bp] read at step tr_off + k; clear: shared [n_hor + 1] */
+    int tr_off;                     /* window offset of this chunk's tracks */
 } ilqg_work;
 
 /* one receding-horizon step of every problem (k_mpc_advance).  The disturbance and the logs are problem-major

@@ -29,7 +29,7 @@ class CuNames:
         kidx = 0
         for d in m.params:
             if d.size == -1:
-                self.map[d.symbols[0]] = f"pk[{kidx}][k]"
+                self.map[d.symbols[0]] = f"pk({kidx}, k)"
                 kidx += 1
             else:
                 for ei, s in enumerate(d.symbols):
@@ -151,7 +151,9 @@ def emit_device(m, struct_name) -> str:
     o.append("    static int param_size(int i) { const int n[] = {%s}; return n[i]; }"
              % ", ".join([str(d.size) for d in m.params] + ["0"]))
     o.append("")
-    ARGS = "const double *p, const double *const *pk, int k, int N, double w_pen, const double *mu"
+    # pk: accessor of the [k]-indexed parameters, pk(j, k) (PkShared / PkTrack in csrc/ilqg_kernels.cuh)
+    ARGS = "const double *p, const PK &pk, int k, int N, double w_pen, const double *mu"
+    TPK = "template <class PK> "
     UNUSED = "        (void)p; (void)pk; (void)k; (void)N; (void)w_pen; (void)mu;"
 
     # ---- rollout step ----------------------------------------------------------------------------------------
@@ -172,16 +174,16 @@ def emit_device(m, struct_name) -> str:
         return render(scA, NR, aux_t) + "\n" + render(scB, NR, aux_t)
 
     o.append("    /* one timestep of the rollout: control already formed in u (pre-clamp); clamps u in place */")
-    o.append(f"    __device__ __forceinline__ static bool step(const double *x, double *u, {ARGS}, double *x_next, double &c) {{")
+    o.append(f"    {TPK}__device__ __forceinline__ static bool step(const double *x, double *u, {ARGS}, double *x_next, double &c) {{")
     o.append("        bool ok = true; double limit; (void)limit;\n" + UNUSED)
     o.append(step_body(False))
     o.append("        return ok;\n    }\n")
     o.append("    /* dynamics and cost of one timestep at the given u, NOT clamped (single evaluations: iLQG_MMex.tem mode 0) */")
-    o.append(f"    __device__ __forceinline__ static bool step_free(const double *x, const double *u, {ARGS}, double *x_next, double &c) {{")
+    o.append(f"    {TPK}__device__ __forceinline__ static bool step_free(const double *x, const double *u, {ARGS}, double *x_next, double &c) {{")
     o.append("        bool ok = true;\n" + UNUSED)
     o.append(step_body(False, clamp=False))
     o.append("        return ok;\n    }\n")
-    o.append(f"    __device__ __forceinline__ static bool step_cost(const double *x, const double *u, {ARGS}, double &c) {{")
+    o.append(f"    {TPK}__device__ __forceinline__ static bool step_cost(const double *x, const double *u, {ARGS}, double &c) {{")
     o.append("        bool ok = true;\n" + UNUSED)
     o.append(step_body(True))
     o.append("        return ok;\n    }\n")
@@ -192,7 +194,7 @@ def emit_device(m, struct_name) -> str:
     for i, e in enumerate(m.g):
         scg.out(("arr", "g", i), e, False)
     o.append(f"    static constexpr int NG = {len(m.g)};")
-    o.append(f"    __device__ __forceinline__ static void calc_g(const double *x, const double *u, {ARGS}, double *g) {{")
+    o.append(f"    {TPK}__device__ __forceinline__ static void calc_g(const double *x, const double *u, {ARGS}, double *g) {{")
     o.append("        (void)x; (void)u; (void)g;\n" + UNUSED)
     o.append(render(scg, NR, aux_t, guards=False) if m.g else "")
     o.append("    }\n")
@@ -201,7 +203,7 @@ def emit_device(m, struct_name) -> str:
     sc = Scope("f")
     aux_outs(sc, m.aux, lambda a: a.used_final)
     sc.out(("c",), m.F, True)
-    o.append(f"    __device__ __forceinline__ static bool final_cost(const double *x, {ARGS}, double &c) {{")
+    o.append(f"    {TPK}__device__ __forceinline__ static bool final_cost(const double *x, {ARGS}, double &c) {{")
     o.append("        bool ok = true;\n" + UNUSED)
     o.append(render(sc, NF, aux_t))
     o.append("        return ok;\n    }\n")
@@ -278,7 +280,7 @@ def emit_device(m, struct_name) -> str:
     o.append("    __device__ __forceinline__ static double dm_inf() { return dm_from_bits(0x7ff0000000000000ull); }\n")
     for full, fname in ((False, "derivs"), (True, "derivs_full")):
         o.append(f"    /* time-varying derivative entries of step k (+ shifted input limits){' incl. second-order dynamics' if full else ''} */")
-        o.append(f"    __device__ __forceinline__ static bool {fname}(const double *x, const double *u, {ARGS}, double *v1, double *v2) {{")
+        o.append(f"    {TPK}__device__ __forceinline__ static bool {fname}(const double *x, const double *u, {ARGS}, double *v1, double *v2) {{")
         o.append("        bool ok = true; double limit; (void)limit; (void)v2;\n" + UNUSED)
         o.append(derivs_body(full))
         o.append("        return ok;\n    }\n")
@@ -291,7 +293,7 @@ def emit_device(m, struct_name) -> str:
         sc.out(("arr", "cx", e.idx), e.expr, not e.atomic and e.time_var)
     for e in m.Fcxx:
         sc.out(("arr", "cxx", e.idx), e.expr, not e.atomic and e.time_var)
-    o.append(f"    __device__ __forceinline__ static bool derivs_final(const double *x, {ARGS}, double *cx, double *cxx) {{")
+    o.append(f"    {TPK}__device__ __forceinline__ static bool derivs_final(const double *x, {ARGS}, double *cx, double *cxx) {{")
     o.append("        bool ok = true;\n" + UNUSED)
     o.append(render(sc, NF, aux_t))
     o.append("        return ok;\n    }\n")
@@ -437,11 +439,11 @@ def emit_device(m, struct_name) -> str:
         return render(sc, NN, aux_t, guards=False)
 
     o.append("    /* constraint values and updated multipliers; is_ineq[i] tells which test update_multipliers applies */")
-    o.append(f"    __device__ __forceinline__ static void mult_running(const double *x, const double *u, {ARGS}, double *hval, double *mu_next) {{")
+    o.append(f"    {TPK}__device__ __forceinline__ static void mult_running(const double *x, const double *u, {ARGS}, double *hval, double *mu_next) {{")
     o.append(UNUSED + "\n        (void)x; (void)u; (void)hval; (void)mu_next;")
     o.append(mult_fn(False))
     o.append("    }")
-    o.append(f"    __device__ __forceinline__ static void mult_final(const double *x, {ARGS}, double *hval, double *mu_next) {{")
+    o.append(f"    {TPK}__device__ __forceinline__ static void mult_final(const double *x, {ARGS}, double *hval, double *mu_next) {{")
     o.append(UNUSED + "\n        (void)x; (void)hval; (void)mu_next;")
     o.append(mult_fn(True))
     o.append("    }")

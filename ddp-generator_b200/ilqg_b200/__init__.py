@@ -69,6 +69,9 @@ class Library:
         L.ilqgb_set_opt.argtypes = [vp, cp, dp, ci]
         L.ilqgb_set_param.argtypes = [vp, ci, dp, ci]
         L.ilqgb_set_param_batch.argtypes = [vp, ci, dp, ci]
+        L.ilqgb_set_param_track.argtypes = [vp, ci, dp, ci]
+        L.ilqgb_set_track_offset.argtypes = [vp, ci]
+        L.ilqgb_track_offset.argtypes = [vp]
         L.ilqgb_validate_opt.restype = cp
         L.ilqgb_validate_opt.argtypes = [cp, dp, ci]
         L.ilqgb_upload.argtypes = [vp, dp, dp]
@@ -168,6 +171,23 @@ class BatchSolver:
             i = self.L.param_names.index(name)
             v = np.ascontiguousarray(np.asarray(val, dtype=np.float64).reshape(self.B, -1))
             self._chk(self.lib.ilqgb_set_param_batch(self.h, i, _ptr(v), v.shape[1]))
+
+    def set_param_track(self, name, values):
+        """A track per problem for the [k]-indexed parameter `name`: values [batch, len], len >= n_hor + 1 (ilqgb_set_param_track).
+        A solve reads name[k] = values[b, offset + k]; shift() and mpc() move the offset with the plan.  set_params() with
+        this name makes the parameter shared again."""
+        i = self.L.param_names.index(name)
+        v = np.ascontiguousarray(np.asarray(values, dtype=np.float64))
+        if v.ndim != 2 or v.shape[0] != self.B:
+            raise ValueError(f"track of '{name}' must be [batch, len] = [{self.B}, >= {self.T + 1}], got {list(v.shape)}")
+        self._chk(self.lib.ilqgb_set_param_track(self.h, i, _ptr(v), v.shape[1]))
+
+    def set_track_offset(self, n):
+        """Window offset of every track: the next solve reads values[b, n + k] (ilqgb_set_track_offset)."""
+        self._chk(self.lib.ilqgb_set_track_offset(self.h, int(n)))
+
+    def track_offset(self):
+        return int(self.lib.ilqgb_track_offset(self.h))
 
     # data ----------------------------------------------------------------------------------------------------------------
     def upload(self, x0, u0):

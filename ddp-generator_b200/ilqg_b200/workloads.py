@@ -72,6 +72,42 @@ def car_batch(B, T=CAR_T, seed=2, first=0):
     return x0, u0
 
 
+# ---- car tracking a reference path (problem cartrack, authored here) -----------------------------------------------------
+CARTRACK_PARAMS = {
+    "d": [2.0], "h": [0.03],
+    "cu": [1e-2 * 1.0, 1e-2 * 0.01], "cx": [1.0, 1.0], "px": [0.1, 0.1], "cf": [1.0, 1.0],
+    "limW": [-0.5, 0.5], "limA": [-2.0, 2.0],
+}
+
+
+def cartrack_batch(B, T=CAR_T, extra=20, seed=4, first=0):
+    """Problems first..first+B-1, each following its own constant-speed arc: speed U(0.5, 2), curvature U(-0.2, 0.2), heading
+    U(0, 2pi), start U(-2, 2)^2, sampled every h = 0.03 s (the car's step).  Returns x0 [B, 4] (near the start of the path,
+    at the path's speed), u0 [B, T, 2] = 0.1*N(0,1) and the tracks {"xr", "yr"}: [B, T + 1 + extra], enough for a closed
+    loop of extra + 1 steps."""
+    b = np.arange(first, first + B, dtype=np.uint64)
+    speed = 0.5 + 1.5 * uniform01(seed, b, 0)
+    kappa = -0.2 + 0.4 * uniform01(seed, b, 1)
+    head = 2.0 * np.pi * uniform01(seed, b, 2)
+    px0 = -2.0 + 4.0 * uniform01(seed, b, 3)
+    py0 = -2.0 + 4.0 * uniform01(seed, b, 4)
+    s = speed[:, None] * (CARTRACK_PARAMS["h"][0] * np.arange(T + 1 + extra))[None, :]     # arc length at each step
+    kap = kappa[:, None]
+    straight = np.abs(kap) < 1e-9
+    ks = np.where(straight, 1.0, kap)
+    th = head[:, None] + kap * s
+    xr = px0[:, None] + np.where(straight, s * np.cos(head)[:, None], (np.sin(th) - np.sin(head)[:, None]) / ks)
+    yr = py0[:, None] + np.where(straight, s * np.sin(head)[:, None], (np.cos(head)[:, None] - np.cos(th)) / ks)
+    x0 = np.zeros((B, 4))
+    x0[:, 0] = px0 + 0.2 * (uniform01(seed, b, 5) - 0.5)
+    x0[:, 1] = py0 + 0.2 * (uniform01(seed, b, 6) - 0.5)
+    x0[:, 2] = head + 0.2 * (uniform01(seed, b, 7) - 0.5)
+    x0[:, 3] = speed
+    idx = np.arange(T * 2, dtype=np.uint64)[None, :] + np.uint64(16)
+    u0 = 0.1 * normal(seed, b[:, None], idx).reshape(B, T, 2)
+    return x0, u0, {"xr": xr, "yr": yr}
+
+
 # ---- brachistochrone ----------------------------------------------------------------------------------------------
 def brachi(n):
     """Config 2 (testBrachi.m:7-22): g=9.81, yf=-4, x0=-eps, u0=-1, dx=2*pi/n; options max_iter=20, w_pen_fact2=2.

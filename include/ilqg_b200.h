@@ -73,6 +73,16 @@ int ilqgb_set_param(ilqgb_handle *h, int index, const double *value, int n);
 /* one value set per problem: value[batch][n].  A batch is then B independent reference calls, each with its own parameter
  * struct (iLQG_mex.c:70-84); parameters never set this way keep the shared value.  Not for [k]-indexed parameters. */
 int ilqgb_set_param_batch(ilqgb_handle *h, int index, const double *value, int n);
+/* Time-indexed parameter tracks.  A [k]-indexed parameter (ilqgb_param_size(index) == -1) gets one track per problem,
+ * value[batch][len] (problem-major, global problem index for multi-device handles), len >= n_hor + 1.  A solve reads
+ * name[k] = track[b][offset + k], k = 0..n_hor.  The handle has ONE window offset for all its tracks: 0 after the first
+ * ilqgb_set_param_track; ilqgb_set_track_offset sets it; ilqgb_shift(n) adds n; ilqgb_mpc adds 1 per shift (n_steps - 1 in
+ * all: the handle keeps the last step's unshifted solution).  ilqgb_upload does not move it.  Any call that would leave a
+ * window past the end of a track fails before doing anything.  ilqgb_set_param on the same index drops the track: the
+ * parameter is shared and fixed again, exactly as today.  [k]-indexed parameters without a track keep today's behaviour. */
+int ilqgb_set_param_track(ilqgb_handle *h, int index, const double *value, int len);
+int ilqgb_set_track_offset(ilqgb_handle *h, int offset);
+int ilqgb_track_offset(const ilqgb_handle *h);
 
 /* host -> device: x0 [batch][nx], u_nom [batch][n_hor][nu] (problem-major, as a caller holds them) */
 int ilqgb_upload(ilqgb_handle *h, const double *x0, const double *u_nom);
@@ -92,7 +102,8 @@ int ilqgb_solve_host(ilqgb_handle *h, const double *x0, const double *u_nom, dou
 int ilqgb_active(ilqgb_handle *h); /* problems still running (synchronises) */
 
 /* Receding horizon.  One closed-loop step is one reference call (upload + solve, every counter, lambda, penalty weight and
- * multiplier re-initialised); [k]-indexed parameters are not shifted.  A problem whose solve failed (result 0 or -1) goes on
+ * multiplier re-initialised); [k]-indexed parameters are not shifted unless they have a track (ilqgb_set_param_track), whose
+ * window then moves with the plan.  A problem whose solve failed (result 0 or -1) goes on
  * with whatever its nominal trajectory holds, as a host loop over ilqgb_solve would.
  * The current solution of every problem becomes the input of the next solve (the reference's caller does this by hand between
  * two iLQG_mex calls): u[k] <- u[k+n_shift] (k < n_hor-n_shift), u[n_hor-1] after that; x0 <- x0 (host [batch][nx]) if given,
