@@ -1122,10 +1122,23 @@ static long ck_get_int(chunk *h, const char *f, int *out)
     else if (!strcmp(f, "n_tails")) scal = w->n_tail;
     else if (!strcmp(f, "bp_done")) scal = w->bp_done;
     else if (!strcmp(f, "deriv_fail")) scal = w->deriv_fail;
-    if (!strcmp(f, "bp_split")) { /* lanes per problem the last backward pass of this chunk ran with (test hook) */
+    {
+        /* test hooks: the kernel variant the last backward pass and line search of this chunk ran with.  bp_split: lanes per
+           problem of the small-batch backward pass (4) or 0; cw_lpp: lanes per problem of the warp-cooperative backward pass, 0
+           for problems that do not use it; bp_latency: register build of k_backpass; ls_tail_from: sequential rounds before
+           the parallel-alpha tail (n_alpha = no tail); ls_commit_par: checkpointed segment-parallel commit (1) or sequential */
+        int v = 0, is_hook = 1;
         size_t b;
-        for (b = 0; b < B; b++) out[b] = h->o.bp_split;
-        return (long)B;
+        if (!strcmp(f, "bp_split")) v = h->o.bp_split;
+        else if (!strcmp(f, "cw_lpp")) v = h->d.coop ? h->o.cw_lpp : 0;
+        else if (!strcmp(f, "bp_latency")) v = h->o.bp_latency_build;
+        else if (!strcmp(f, "ls_tail_from")) v = h->o.ls_tail_from;
+        else if (!strcmp(f, "ls_commit_par")) v = h->o.ls_commit_par;
+        else is_hook = 0;
+        if (is_hook) {
+            for (b = 0; b < B; b++) out[b] = v;
+            return (long)B;
+        }
     }
     if (scal) {
         if (ilqgk_d2h(out, scal, sizeof(int) * B, h->stream) || ilqgk_stream_sync(h->stream)) return failk(h);

@@ -21,7 +21,8 @@ LIB_DIR = os.environ.get("ILQG_LIB_DIR") or os.path.join(os.path.dirname(_HERE),
 TRACE, TIMING = 1, 2
 KERNEL_CLASSES = ("derivs", "backpass", "linesearch", "post")
 _SCALAR_FIELDS = {"cost", "new_cost", "dcost", "expected", "lambda", "dlambda", "g_norm", "dV0", "dV1", "w_pen_l", "w_pen_f",
-                  "iterations", "result", "status", "n_linesearch", "n_backpass", "n_derivs", "n_rollouts", "n_tails", "cur", "bp_split"}
+                  "iterations", "result", "status", "n_linesearch", "n_backpass", "n_derivs", "n_rollouts", "n_tails", "cur", "bp_split",
+                  "cw_lpp", "bp_latency", "ls_tail_from", "ls_commit_par"}
 
 
 def lib_path(problem, full_ddp, lib_dir=None):

@@ -166,7 +166,11 @@ int ilqgb_set_tuning(ilqgb_handle *h, const char *name, int value);
  * have been re-evaluated at its final trajectory by a later sweep (they are never read again by the solver). */
 long ilqgb_get(ilqgb_handle *h, const char *field, double *out);
 /* "iterations" "result" "status" "n_linesearch" "n_backpass" "n_derivs" "n_rollouts" "n_tails" "cur" "bp_done" "deriv_fail" -> [batch]; "tr_alpha" -> [batch][max_iter];
- * "tr_clamp" -> [batch][n_hor] (2 bits per input: 0 free, 1 lower, 2 upper; QP return code in bits 16..23) */
+ * "tr_clamp" -> [batch][n_hor] (2 bits per input: 0 free, 1 lower, 2 upper; QP return code in bits 16..23);
+ * the kernel variants the last pass ran with, the same value for every problem of a chunk -> [batch]: "bp_split" (4 or 0),
+ * "cw_lpp" (lanes per problem of the warp-cooperative backward pass, 0 where the problem does not use it), "bp_latency"
+ * (register build of the lane-per-problem backward pass), "ls_tail_from" (sequential line-search rounds before the tail,
+ * n_alpha = none), "ls_commit_par" (1 = checkpointed segment-parallel commit, 0 = sequential; ILQG_LS_COMMIT_PAR) */
 long ilqgb_get_int(ilqgb_handle *h, const char *field, int *out);
 
 /* host -> device write of a field (names and shapes of ilqgb_get, plus "x0" "x_cand" "u_cand" "last_r" "last_f";
