@@ -91,6 +91,8 @@ template <bool PP> static int preload_pp()
     return bad;
 }
 
+constexpr bool HAS_KP = P::NKP > 0;
+
 extern "C" {
 
 const char *ilqgk_last_error(void) { return g_err; }
@@ -105,6 +107,8 @@ int ilqgk_preload(void)
     bad |= split_launcher<P, false, SPLIT_OK>::preload() | split_launcher<P, true, SPLIT_OK>::preload();
     bad |= preload_one(k_finalize) | preload_one(k_count_active) | preload_one(k_scatter) | preload_one(k_gather);
     bad |= preload_one(k_mpc_advance<P>);   /* first launched between two steps of a closed loop, while other chunks solve */
+    bad |= preload_one(k_mpc_plant<P, false, false>) | preload_one(k_mpc_plant<P, true, false>);
+    if constexpr (HAS_KP) bad |= preload_one(k_mpc_plant<P, false, true>) | preload_one(k_mpc_plant<P, true, true>);
     if (bad) { snprintf(g_err, sizeof g_err, "loading the kernels failed: %s", cudaGetErrorString(cudaGetLastError())); return -1; }
     if (dev >= 0 && dev < ILQGK_MAX_DEVICES) loaded[dev] = 1;
     return 0;
@@ -176,7 +180,6 @@ static inline unsigned nblk(int n, int bs) { return (unsigned)((n + bs - 1) / bs
     } while (0)
 /* the kernels that evaluate the problem functions also exist, for problems with [k]-indexed parameters, in a variant that
    reads per-problem tracks (TR); without such parameters both branches name the same instantiation */
-constexpr bool HAS_KP = P::NKP > 0;
 #define PK_DISPATCH(w_, CALL)                                                                                         \
     do {                                                                                                              \
         if (HAS_KP && (w_)->tr_mask) { constexpr bool TR = HAS_KP; PP_DISPATCH(w_, CALL); }                            \
@@ -366,6 +369,22 @@ int ilqgk_launch_mpc_advance(const ilqg_work *w, const ilqg_mpc_step *a, void *s
 {
     k_mpc_advance<P><<<nblk(w->B, 256), 256, 0, (cudaStream_t)stream>>>(*w, *a);
     return check(cudaGetLastError(), "k_mpc_advance");
+}
+
+int ilqgk_launch_mpc_plant(const ilqg_work *w, const ilqg_mpc_step *a, const double *params_plant, const ilqg_plant *pl, void *stream)
+{
+    /* PPP: per-problem plant table; TR: the model's [k]-indexed parameters from the tracks */
+    const ParamBlock<P> pb = make_pb(params_plant);
+    const unsigned grid = nblk(w->B, 256);
+    if (HAS_KP && w->tr_mask) {
+        constexpr bool TR = HAS_KP;
+        if (pl->pp) k_mpc_plant<P, true, TR><<<grid, 256, 0, (cudaStream_t)stream>>>(*w, *a, pb, *pl);
+        else k_mpc_plant<P, false, TR><<<grid, 256, 0, (cudaStream_t)stream>>>(*w, *a, pb, *pl);
+    } else {
+        if (pl->pp) k_mpc_plant<P, true, false><<<grid, 256, 0, (cudaStream_t)stream>>>(*w, *a, pb, *pl);
+        else k_mpc_plant<P, false, false><<<grid, 256, 0, (cudaStream_t)stream>>>(*w, *a, pb, *pl);
+    }
+    return check(cudaGetLastError(), "k_mpc_plant");
 }
 
 int ilqgk_launch_scatter(const double *src, double *dst, double *dst_alt, const int *sel, int B, int n_k, int n_i, long long stride_k,

@@ -64,6 +64,8 @@ int ilqgk_launch_finalize(const ilqg_work *w, int max_iter, void *stream);
 int ilqgk_launch_count_active(const ilqg_work *w, int *d_counter, void *stream);
 /* log the finished solve of every problem and shift its solution into the input of the next one (k_mpc_advance) */
 int ilqgk_launch_mpc_advance(const ilqg_work *w, const ilqg_mpc_step *a, void *stream);
+/* the same with the next state from the plant (k_mpc_plant): params_plant = the shared plant set (used when pl->pp is null) */
+int ilqgk_launch_mpc_plant(const ilqg_work *w, const ilqg_mpc_step *a, const double *params_plant, const ilqg_plant *pl, void *stream);
 /* [B][n_k][n_i] (host order) <-> device element (k, b, i) at base[k*stride_k + b*stride_b + i*stride_i + off] */
 int ilqgk_launch_scatter(const double *src, double *dst, double *dst_alt, const int *sel, int B, int n_k, int n_i, long long stride_k,
                          long long stride_b, long long stride_i, long long off, void *stream);

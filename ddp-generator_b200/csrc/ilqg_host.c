@@ -40,6 +40,15 @@ struct chunk {
                               their window offset is w.tr_off and their bits are w.tr_mask */
     int tr_len[16];
     double *d_pp;          /* per-problem parameter sets [npf][Bp] (ilqg_work.pp), allocated on first use */
+    /* plant of the closed loops (ilqgb_set_plant_*): per flat parameter entry, where its value comes from; the plant's shared
+       values; its per-problem values [npf][Bp]; and the table k_mpc_plant reads, rebuilt when anything it depends on changed */
+    int plant_on, plant_n_sub, plant_dirty;
+    unsigned char *plant_src;   /* [npf] PLANT_MODEL, PLANT_SHARED or PLANT_BATCH */
+    double *plant_val;          /* [npf] shared plant values */
+    double *d_plant_pp;         /* [npf][Bp] per-problem plant values (rows of PLANT_BATCH entries), allocated on first use */
+    double *plant_params;       /* [npf] effective shared set (when neither the model nor the plant is per-problem) */
+    double *d_plant_eff;        /* [npf][Bp] effective per-problem set, allocated on first use */
+    int plant_per;              /* the effective set is d_plant_eff (else plant_params) */
     void *stream;          /* the stream all work of this chunk is enqueued on (stream_main, or stream_io during an end-to-end solve) */
     void *stream_main, *stream_io;
     int owns_stream;
@@ -73,6 +82,8 @@ struct chunk {
     long n_launches;       /* kernels launched since creation */
     char err[256];
 };
+
+enum { PLANT_MODEL = 0, PLANT_SHARED = 1, PLANT_BATCH = 2 };
 
 static char g_create_err[256] = "";
 #define fail_create(msg) (snprintf(g_create_err, sizeof g_create_err, "%s", msg), (void)0)
@@ -266,18 +277,21 @@ static int param_offset(int index)
     return off;
 }
 
-/* one row [Bp] of the per-problem table = the same value for every problem */
-static int pp_fill_row(chunk *h, int row, double v)
+/* one device row [Bp] = the same value for every problem */
+static int fill_row(chunk *h, double *dst, double v)
 {
     size_t b;
     double *tmp = (double *)malloc(sizeof(double) * h->Bp);
     int rc;
     if (!tmp) return fail(h, "out of host memory");
     for (b = 0; b < (size_t)h->Bp; b++) tmp[b] = v;
-    rc = ilqgk_h2d(h->d_pp + (size_t)row * h->Bp, tmp, sizeof(double) * h->Bp, h->stream) || ilqgk_stream_sync(h->stream);
+    rc = ilqgk_h2d(dst, tmp, sizeof(double) * h->Bp, h->stream) || ilqgk_stream_sync(h->stream);
     free(tmp);
     return rc ? failk(h) : 0;
 }
+
+/* one row of the per-problem table = the same value for every problem */
+static int pp_fill_row(chunk *h, int row, double v) { return fill_row(h, h->d_pp + (size_t)row * h->Bp, v); }
 
 /* parameter `index` for every problem of the chunk: value[b][n] (a batch of independent reference calls, each with
    its own parameter struct).  The first call switches the chunk to per-problem parameters, seeded from the shared set. */
@@ -290,6 +304,7 @@ static int ck_set_param_batch(chunk *h, int index, const double *value, int n)
     if (ilqgk_param_size(index) == -1) return fail(h, "[k]-indexed parameters are shared by the batch");
     if (n != ilqgk_param_size(index)) return fail(h, "wrong parameter length");
     if (ilqgk_set_device(h->device)) return failk(h);
+    h->plant_dirty = 1;   /* plant entries that follow the model follow this change */
     if (!h->d_pp) {
         h->d_pp = (double *)dalloc(h, sizeof(double) * (size_t)(h->d.npf > 0 ? h->d.npf : 1) * h->Bp);
         if (!h->d_pp) return -1;
@@ -375,9 +390,111 @@ static int ck_set_param(chunk *h, int index, const double *value, int n)
     for (i = 0; i < index; i++)
         if (ilqgk_param_size(i) > 0) off += ilqgk_param_size(i);
     memcpy(h->params + off, value, sizeof(double) * n);
+    h->plant_dirty = 1;
     if (h->d_pp) /* per-problem table in use: a shared value overwrites every problem's entry */
         for (i = 0; i < n; i++)
             if (pp_fill_row(h, off + i, value[i])) return -1;
+    return 0;
+}
+
+/* ---- plant of the closed loops (see ilqg_b200.h); index, value and length are checked by the caller ---- */
+static void ck_set_plant_param(chunk *h, int index, const double *value, int n)
+{
+    const int off = param_offset(index);
+    int i;
+    for (i = 0; i < n; i++) {
+        h->plant_src[off + i] = PLANT_SHARED;
+        h->plant_val[off + i] = value[i];
+    }
+    h->plant_on = 1;
+    h->plant_dirty = 1;
+}
+
+static int ck_set_plant_param_batch(chunk *h, int index, const double *value, int n)
+{
+    const int off = param_offset(index);
+    int i;
+    size_t b;
+    double *tmp;
+    if (ilqgk_set_device(h->device)) return failk(h);
+    if (!h->d_plant_pp) {
+        h->d_plant_pp = (double *)dalloc(h, sizeof(double) * (size_t)h->d.npf * h->Bp);
+        if (!h->d_plant_pp) return -1;
+    }
+    tmp = (double *)calloc((size_t)h->Bp, sizeof(double));
+    if (!tmp) return fail(h, "out of host memory");
+    for (i = 0; i < n; i++) {
+        for (b = 0; b < (size_t)h->B; b++) tmp[b] = value[b * n + i];
+        if (ilqgk_h2d(h->d_plant_pp + (size_t)(off + i) * h->Bp, tmp, sizeof(double) * h->Bp, h->stream) || ilqgk_stream_sync(h->stream)) {
+            free(tmp);
+            return failk(h);
+        }
+        h->plant_src[off + i] = PLANT_BATCH;
+    }
+    free(tmp);
+    h->plant_on = 1;
+    h->plant_dirty = 1;
+    return 0;
+}
+
+static void ck_clear_plant(chunk *h)
+{
+    ilqgk_set_device(h->device);
+    dfree(h, h->d_plant_pp);   /* cudaFree waits for the work that still reads it */
+    dfree(h, h->d_plant_eff);
+    h->d_plant_pp = h->d_plant_eff = NULL;
+    memset(h->plant_src, PLANT_MODEL, (size_t)(h->d.npf > 0 ? h->d.npf : 1));
+    h->plant_on = h->plant_per = 0;
+    h->plant_n_sub = 1;
+    h->plant_dirty = 1;
+}
+
+/* The one table k_mpc_plant reads, entry by entry the plant's own value where it has one and the model's current value
+   (shared, or this problem's under per-problem model parameters) elsewhere.  A shared set when neither the model nor the
+   plant is per-problem, else [npf][Bp] built on the device.  Rebuilt only after a change (plant_dirty). */
+static int ck_plant_prepare(chunk *h)
+{
+    const size_t Bp = (size_t)h->Bp;
+    int i, per = h->d_pp != NULL;
+    if (!h->plant_dirty) return 0;
+    for (i = 0; i < h->d.npf; i++) {
+        h->plant_params[i] = h->plant_src[i] == PLANT_SHARED ? h->plant_val[i] : h->params[i];
+        if (h->plant_src[i] == PLANT_BATCH) per = 1;
+    }
+    if (per) {
+        if (ilqgk_set_device(h->device)) return failk(h);
+        if (!h->d_plant_eff) {
+            h->d_plant_eff = (double *)dalloc(h, sizeof(double) * (size_t)h->d.npf * Bp);
+            if (!h->d_plant_eff) return -1;
+        }
+        for (i = 0; i < h->d.npf; i++) {
+            double *dst = h->d_plant_eff + (size_t)i * Bp;
+            if (h->plant_src[i] == PLANT_BATCH) {
+                if (ilqgk_d2d(dst, h->d_plant_pp + (size_t)i * Bp, sizeof(double) * Bp, h->stream)) return failk(h);
+            } else if (h->plant_src[i] == PLANT_MODEL && h->d_pp) {
+                if (ilqgk_d2d(dst, h->d_pp + (size_t)i * Bp, sizeof(double) * Bp, h->stream)) return failk(h);
+            } else if (fill_row(h, dst, h->plant_params[i]))
+                return -1;
+        }
+        if (ilqgk_stream_sync(h->stream)) return failk(h);
+    }
+    h->plant_per = per;
+    h->plant_dirty = 0;
+    return 0;
+}
+
+/* x0 of the next solve from the solution's prediction (k_mpc_advance) or, with a plant, from the plant (k_mpc_plant) */
+static int launch_advance(chunk *h, const ilqg_mpc_step *a)
+{
+    if (h->plant_on && a->set_x0) {
+        ilqg_plant pl;
+        if (ck_plant_prepare(h)) return -1;
+        pl.n_sub = h->plant_n_sub;
+        pl.pp = h->plant_per ? h->d_plant_eff : NULL;
+        if (ilqgk_launch_mpc_plant(&h->w, a, h->plant_params, &pl, h->stream)) return failk(h);
+    } else if (ilqgk_launch_mpc_advance(&h->w, a, h->stream))
+        return failk(h);
+    h->n_launches++;
     return 0;
 }
 
@@ -437,6 +554,20 @@ static chunk *ck_create(int device, int batch, int n_hor, int flags, void *strea
         free(h);
         return NULL;
     }
+    h->plant_src = (unsigned char *)calloc((size_t)(h->d.npf > 0 ? h->d.npf : 1), 1);
+    h->plant_val = (double *)calloc((size_t)(h->d.npf > 0 ? h->d.npf : 1), sizeof(double));
+    h->plant_params = (double *)calloc((size_t)(h->d.npf > 0 ? h->d.npf : 1), sizeof(double));
+    if (!h->plant_src || !h->plant_val || !h->plant_params) {
+        fail(NULL, "out of host memory");
+        free(h->plant_src);
+        free(h->plant_val);
+        free(h->plant_params);
+        free(h->params);
+        free(h);
+        return NULL;
+    }
+    h->plant_n_sub = 1;
+    h->plant_dirty = 1;
     ck_standard_parameters(h);
     h->prio_rank = prio_rank;
     h->prio_n = prio_n;
@@ -556,6 +687,9 @@ static void ck_destroy(chunk *h)
     if (h->stream_io) ilqgk_stream_destroy(h->stream_io);
     if (h->owns_stream && h->stream_main) ilqgk_stream_destroy(h->stream_main);
     free(h->params);
+    free(h->plant_src);
+    free(h->plant_val);
+    free(h->plant_params);
     free(h);
 }
 
@@ -642,8 +776,7 @@ static int ck_shift(chunk *h, int n_shift, const double *x0, const double *w)
         if (ilqgk_h2d(h->d_stage, w, sizeof(double) * B * nx, h->stream)) return failk(h);
         a.w = h->d_stage;
     }
-    if (ilqgk_launch_mpc_advance(&h->w, &a, h->stream)) return failk(h);
-    h->n_launches++;
+    if (launch_advance(h, &a)) return -1;
     if (x0) { /* into its own [NX][Bp] array, as ck_upload does */
         if (ilqgk_h2d(h->d_stage, x0, sizeof(double) * B * nx, h->stream)) return failk(h);
         if (ilqgk_launch_scatter(h->d_stage, h->w.x0, NULL, NULL, h->B, 1, h->d.nx, 0, 1, h->Bp, 0, h->stream)) return failk(h);
@@ -670,6 +803,7 @@ static int ck_mpc_begin(chunk *h, const mpc_t *m, const double *w)
     const size_t n_it = m->iterations ? ints : 0, n_res = m->result ? ints : 0;
     double *s;
     if (ilqgk_set_device(h->device)) return failk(h);
+    if (h->plant_on && ck_plant_prepare(h)) return -1;   /* here, not between two steps of the loop */
     if (ensure_stage(h, n_w + n_x + n_u + n_c + n_it + n_res)) return -1;
     s = h->d_stage;
     memset(&h->mpc, 0, sizeof h->mpc);
@@ -698,8 +832,7 @@ static int ck_mpc_advance(chunk *h, int step)
 {
     h->mpc.step = step;
     h->mpc.plan = step + 1 < h->mpc.n_steps;
-    if (ilqgk_launch_mpc_advance(&h->w, &h->mpc, h->stream)) return failk(h);
-    h->n_launches++;
+    if (launch_advance(h, &h->mpc)) return -1;
     if (h->mpc.plan) {
         h->started = 0;   /* the input has been replaced */
         h->w.tr_off++;    /* the tracks move with the plan: every later launch of this chunk passes the next window */
@@ -1071,6 +1204,18 @@ static long ck_get(chunk *h, const char *f, double *out)
             return failk(h);
         h->n_launches++;
         return (long)n;
+    }
+    if (!strcmp(f, "plant")) { /* computed field: the effective plant parameter set of every problem [B][npf] */
+        const size_t npf = (size_t)h->d.npf;
+        size_t b;
+        if (ck_plant_prepare(h)) return -1;
+        if (!h->plant_per) {
+            for (b = 0; b < B; b++) memcpy(out + b * npf, h->plant_params, sizeof(double) * npf);
+            return (long)(B * npf);
+        }
+        if (gather_to_host(h, h->d_plant_eff, NULL, NULL, 1, h->d.npf, lay_soa(h, h->d.npf), out)) return -1;
+        if (ilqgk_stream_sync(h->stream)) return failk(h);
+        return (long)(B * npf);
     }
     if (find_field(h, f, &fd)) return -1;
     if (fd.scal) {
@@ -1457,6 +1602,53 @@ int ilqgb_set_track_offset(ilqgb_handle *h, int offset)
 }
 
 int ilqgb_track_offset(const ilqgb_handle *h) { return h->tr_off; }
+
+/* ---- plant of the closed loops (see ilqg_b200.h) ---- */
+static int plant_param_ok(ilqgb_handle *h, int index, const double *value, int n)
+{
+    const char *msg = NULL;
+    if (index < 0 || index >= ilqgk_param_count()) msg = "parameter index out of range";
+    else if (ilqgk_param_size(index) == -1) msg = "[k]-indexed parameters of the plant are the model's: they cannot be set";
+    else if (n != ilqgk_param_size(index)) msg = "wrong parameter length";
+    else if (!value) msg = "no parameter values";
+    if (msg) snprintf(h->err, sizeof h->err, "%s", msg);
+    return !msg;
+}
+
+int ilqgb_set_plant_param(ilqgb_handle *h, int index, const double *value, int n)
+{
+    int i;
+    if (!plant_param_ok(h, index, value, n)) return -1;
+    for (i = 0; i < h->n; i++) ck_set_plant_param(h->c[i], index, value, n);
+    return 0;
+}
+
+int ilqgb_set_plant_param_batch(ilqgb_handle *h, int index, const double *value, int n)
+{
+    int i;
+    if (!plant_param_ok(h, index, value, n)) return -1;
+    for (i = 0; i < h->n; i++)
+        if (ck_set_plant_param_batch(h->c[i], index, value + (size_t)h->first[i] * n, n)) return hfail(h, h->c[i]);
+    return 0;
+}
+
+int ilqgb_set_plant_substeps(ilqgb_handle *h, int n_sub)
+{
+    int i;
+    if (n_sub < 1 || n_sub > 64) { snprintf(h->err, sizeof h->err, "n_sub must be in 1..64"); return -1; }
+    for (i = 0; i < h->n; i++) {
+        h->c[i]->plant_n_sub = n_sub;
+        h->c[i]->plant_on = 1;
+    }
+    return 0;
+}
+
+int ilqgb_clear_plant(ilqgb_handle *h)
+{
+    int i;
+    for (i = 0; i < h->n; i++) ck_clear_plant(h->c[i]);
+    return 0;
+}
 
 int ilqgb_upload(ilqgb_handle *h, const double *x0, const double *u_nom)
 {

@@ -2131,23 +2131,16 @@ __global__ void k_count_active(Work w, int *out)
  * them and k_init's initial rollout reads them, and x[n_shift] (+ w) becomes x0.  Whatever the nominal buffer holds is
  * used, also for a problem whose solve failed.  When cur[b] == 0 the source is the destination: every record is read before
  * it is written because the steps are copied in ascending order, KB of them loaded before any is stored (a copy parallel
- * over (k, b) would not be safe).  Adjacent threads are adjacent problems of the [k][Bp][RXU] records. */
+ * over (k, b) would not be safe).  Adjacent threads are adjacent problems of the [k][Bp][RXU] records.
+ * mpc_log_shift is everything after the next state xn (+ w) is known; k_mpc_advance and k_mpc_plant differ only in how
+ * they compute xn. */
 template <class P>
-__global__ void __launch_bounds__(256) k_mpc_advance(Work w, ilqg_mpc_step a)
+__device__ __forceinline__ void mpc_log_shift(const Work &w, const ilqg_mpc_step &a, int b, const double *src, const double *xn)
 {
     constexpr int NX = P::NX, NU = P::NU, RXU = Rec<P>::RXU, KB = 8;
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= w.B) return;
     const size_t Bp = w.Bp;
     const int T = w.T, n = a.n_shift;
-    const double *src = w.XU[w.cur[b]];
     const size_t row = (size_t)b * a.n_steps + a.step;
-    double xn[NX];
-#pragma unroll
-    for (int i = 0; i < NX; i++) {
-        xn[i] = src[((size_t)n * Bp + b) * RXU + i];
-        if (a.w) xn[i] = xn[i] + a.w[row * NX + i];
-    }
     if (a.x_log) {
         double *xl = a.x_log + ((size_t)b * (a.n_steps + 1) + a.step) * NX;
 #pragma unroll
@@ -2182,6 +2175,69 @@ __global__ void __launch_bounds__(256) k_mpc_advance(Work w, ilqg_mpc_step a)
 #pragma unroll
                 for (int i = 0; i < NU; i++) dst[((size_t)(k0 + j) * Bp + b) * RXU + NX + i] = u[j][i];
     }
+}
+
+template <class P>
+__global__ void __launch_bounds__(256) k_mpc_advance(Work w, ilqg_mpc_step a)
+{
+    constexpr int NX = P::NX, RXU = Rec<P>::RXU;
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= w.B) return;
+    const size_t Bp = w.Bp;
+    const int n = a.n_shift;
+    const double *src = w.XU[w.cur[b]];
+    const size_t row = (size_t)b * a.n_steps + a.step;
+    double xn[NX];
+#pragma unroll
+    for (int i = 0; i < NX; i++) {
+        xn[i] = src[((size_t)n * Bp + b) * RXU + i];
+        if (a.w) xn[i] = xn[i] + a.w[row * NX + i];
+    }
+    mpc_log_shift<P>(w, a, b, src, xn);
+}
+
+/* k_mpc_advance against a plant that differs from the model: the next state is not the solution's prediction x[n_shift] but
+ * the plant stepped from the solve's x0 through the n_shift applied controls u[j], each held for pl.n_sub sub-steps.  A sub-step
+ * is P::step -- clampU with the plant's limits at the sub-step's own state, then f -- on a fresh copy of the commanded u[j],
+ * exactly the reference's forward_pass step (and MMex modes 16 then 0), with zero multipliers and penalty weight as in k_clamp.
+ * All sub-steps of control j evaluate at step index j, [k]-indexed parameters from the model (TR: the window of the solve that
+ * just finished).  The plant's parameters: the shared block pb_plant, or (PPP) this problem's column of pl.pp.  A non-finite
+ * state is passed on as it is; the next solve's initial rollout then fails for that problem alone. */
+template <class P, bool PPP, bool TR = false>
+__global__ void __launch_bounds__(256) k_mpc_plant(Work w, ilqg_mpc_step a, ParamBlock<P> pb_plant, ilqg_plant pl)
+{
+    constexpr int NX = P::NX, NU = P::NU, RXU = Rec<P>::RXU;
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= w.B) return;
+    const size_t Bp = w.Bp;
+    double pl_[PPP ? P::NPF : 1];
+    const double *pv = pb_plant.v;
+    if (PPP) {
+#pragma unroll
+        for (int i = 0; i < P::NPF_USED; i++) pl_[i] = pl.pp[(size_t)i * Bp + b];
+        pv = pl_;
+    }
+    ILQG_PK(TR, b)
+    const double *src = w.XU[w.cur[b]];
+    double xn[NX], x[NX], u[NU], mu[P::N_MU_R + P::N_MU_F + 1], c;
+#pragma unroll
+    for (int i = 0; i < NX; i++) xn[i] = w.x0[(size_t)i * Bp + b];
+#pragma unroll
+    for (int i = 0; i < P::N_MU_R; i++) mu[i] = 0.0;
+    for (int j = 0; j < a.n_shift; j++)
+        for (int s = 0; s < pl.n_sub; s++) {
+#pragma unroll
+            for (int i = 0; i < NX; i++) x[i] = xn[i];
+#pragma unroll
+            for (int i = 0; i < NU; i++) u[i] = src[((size_t)j * Bp + b) * RXU + NX + i];
+            P::step(x, u, pv, pk, j, w.T, 0.0, mu, xn, c);
+        }
+    if (a.w) {
+        const size_t row = (size_t)b * a.n_steps + a.step;
+#pragma unroll
+        for (int i = 0; i < NX; i++) xn[i] = xn[i] + a.w[row * NX + i];
+    }
+    mpc_log_shift<P>(w, a, b, src, xn);
 }
 
 /* layout changes between the caller's problem-major arrays [B][n_k][n_i] and device arrays addressed as

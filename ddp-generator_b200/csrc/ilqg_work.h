@@ -67,4 +67,12 @@ typedef struct ilqg_mpc_step {
     int *it_log, *res_log;              /* iterations, result */
 } ilqg_mpc_step;
 
+/* the plant of a closed loop (k_mpc_plant): the same problem with its own parameter values, stepped n_sub times per applied
+ * control.  It travels in k_mpc_plant's own arguments so that ilqg_work and ilqg_mpc_step, which other kernels take by
+ * value, keep their layout. */
+typedef struct ilqg_plant {
+    int n_sub;          /* 1..64 sub-steps per control interval */
+    const double *pp;   /* per-problem plant parameter sets [NPF][Bp], or null = one shared set (kernel argument) */
+} ilqg_plant;
+
 #endif

@@ -71,6 +71,10 @@ class Library:
         L.ilqgb_set_param.argtypes = [vp, ci, dp, ci]
         L.ilqgb_set_param_batch.argtypes = [vp, ci, dp, ci]
         L.ilqgb_set_param_track.argtypes = [vp, ci, dp, ci]
+        L.ilqgb_set_plant_param.argtypes = [vp, ci, dp, ci]
+        L.ilqgb_set_plant_param_batch.argtypes = [vp, ci, dp, ci]
+        L.ilqgb_set_plant_substeps.argtypes = [vp, ci]
+        L.ilqgb_clear_plant.argtypes = [vp]
         L.ilqgb_set_track_offset.argtypes = [vp, ci]
         L.ilqgb_track_offset.argtypes = [vp]
         L.ilqgb_validate_opt.restype = cp
@@ -190,6 +194,40 @@ class BatchSolver:
     def track_offset(self):
         return int(self.lib.ilqgb_track_offset(self.h))
 
+    # plant of the closed loops -------------------------------------------------------------------------------------------
+    def _param_index(self, name):
+        if name not in self.L.param_names:
+            raise KeyError(f"Parameter name '{name}' is not member of parameters struct.")
+        return self.L.param_names.index(name)
+
+    def set_plant_params(self, params):
+        """The plant's own shared values {name: value} (ilqgb_set_plant_param); names not given follow the model.  With a plant,
+        shift() and mpc() step the next x0 from the solve's x0 through the applied controls with these parameters instead of
+        taking the solution's prediction.  [k]-indexed parameters are always the model's."""
+        for name, val in params.items():
+            v = np.ascontiguousarray(np.asarray(val, dtype=np.float64).ravel())
+            self._chk(self.lib.ilqgb_set_plant_param(self.h, self._param_index(name), _ptr(v), v.size))
+
+    def set_plant_params_batch(self, params):
+        """Per-problem plant values {name: array [batch, size]} (ilqgb_set_plant_param_batch)."""
+        for name, val in params.items():
+            i = self._param_index(name)
+            size = self.L.param_sizes[i]
+            v = np.ascontiguousarray(np.asarray(val, dtype=np.float64))
+            if v.ndim == 1 and size == 1:
+                v = v[:, None]
+            if v.shape != (self.B, size):
+                raise ValueError(f"plant values of '{name}' must be [batch, size] = [{self.B}, {size}], got {list(v.shape)}")
+            self._chk(self.lib.ilqgb_set_plant_param_batch(self.h, i, _ptr(v), size))
+
+    def set_plant_substeps(self, n_sub):
+        """Plant steps per control interval, 1..64.  Nothing is rescaled: set the plant's time step to the model's / n_sub."""
+        self._chk(self.lib.ilqgb_set_plant_substeps(self.h, int(n_sub)))
+
+    def clear_plant(self):
+        """No plant: the next x0 is the solution's prediction x[n] (+ w) again."""
+        self._chk(self.lib.ilqgb_clear_plant(self.h))
+
     # data ----------------------------------------------------------------------------------------------------------------
     def upload(self, x0, u0):
         x0 = np.ascontiguousarray(x0, dtype=np.float64)
@@ -295,6 +333,7 @@ class BatchSolver:
 
     # read-back ---------------------------------------------------------------------------------------------------------
     def get(self, field):
+        """A per-problem field of ilqgb_get; "plant" is the effective plant parameter set [B, sum of parameter sizes]."""
         T, nx, nu, B = self.T, self.nx, self.nu, self.B
         nq = nx * (nx + 1) // 2
         shapes = {"x": (B, T + 1, nx), "u": (B, T, nu), "l": (B, T, nu), "L": (B, T, nu * nx), "fd": (B, nx + nq)}

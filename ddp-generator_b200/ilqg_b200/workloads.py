@@ -42,6 +42,27 @@ def disturbance(B, S, nx, scale, seed, first=0):
     return scale * normal(seed, b[:, None], idx).reshape(B, S, nx)
 
 
+def _scaled(seed, b, idx, nominal, spread):
+    """nominal values scaled by U(1 - spread, 1 + spread), one factor per problem b and element idx"""
+    return np.asarray(nominal)[None, :] * (1.0 + spread * (2.0 * uniform01(seed, b[:, None], idx[None, :]) - 1.0))
+
+
+def car_plant(B, spread, seed, first=0):
+    """Sampled car plants for a robustness study: {"d": [B, 1]}, the wheelbase scaled by U(1 - spread, 1 + spread); problems
+    first..first+B-1 (BatchSolver.set_plant_params_batch)."""
+    b = np.arange(first, first + B, dtype=np.uint64)
+    return {"d": _scaled(seed, b, np.arange(1, dtype=np.uint64), CAR_PARAMS["d"], spread)}
+
+
+def quad_plant(B, spread, seed, first=0):
+    """Sampled quadrotor plants: mass [B, 1], inertia J [B, 3] and rotor torque coefficient kq [B, 1], each entry scaled by its
+    own U(1 - spread, 1 + spread); problems first..first+B-1."""
+    b = np.arange(first, first + B, dtype=np.uint64)
+    e = np.arange(5, dtype=np.uint64)
+    return {"mass": _scaled(seed, b, e[:1], QUAD_PARAMS["mass"], spread), "J": _scaled(seed, b, e[1:4], QUAD_PARAMS["J"], spread),
+            "kq": _scaled(seed, b, e[4:], QUAD_PARAMS["kq"], spread)}
+
+
 # ---- car parking ---------------------------------------------------------------------------------------------
 CAR_PARAMS = {
     "d": [2.0], "h": [0.03],

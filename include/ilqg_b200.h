@@ -20,6 +20,8 @@
  *   ilqgb_download                 copy-out of x, u, cost, iLQG_mex.c:127-137, plus iterations / return value
  *   ilqgb_shift / ilqgb_mpc        what a receding-horizon caller does between two iLQG_mex calls (SURVEY.md:211: the
  *                                  previous u, shifted, is the next u_nom), on the device; ilqgb_mpc runs whole closed loops
+ *   ilqgb_set_plant_*              the plant of such a loop, which the caller steps with iLQG<Name>MMex modes 16 and 0 and
+ *                                  the plant's parameter struct (iLQG_MMex.tem:81-226)
  *   ilqgb_phase_*                  calc_derivs / back_pass / line_search on their own (iLQG.h:83, back_pass.h:7,
  *                                  line_search.h:6) for phase-level parity tests
  *   ilqgb_get / ilqgb_get_int      read-back of any per-problem field (tOptSet / trajEl_t members)
@@ -117,6 +119,27 @@ int ilqgb_shift(ilqgb_handle *h, int n_shift, const double *x0, const double *w)
  * ilqgb_download / ilqgb_get return the final plan.  Every chunk advances through the steps on its own.  Synchronises. */
 int ilqgb_mpc(ilqgb_handle *h, int n_steps, const double *x0, const double *u_nom, const double *w,
               double *x_cl, double *u_cl, double *cost, int *iterations, int *result);
+/* A plant that differs from the model (Monte-Carlo robustness of one controller over sampled plants).  The plant is the same
+ * generated problem with its own parameter values, stepped n_sub times per control interval.  With a plant, wherever
+ * ilqgb_shift (without a host x0) and ilqgb_mpc set x0 <- x[n] (+ w), they instead step xp = the finished solve's x0 through the
+ * n applied controls u[j], j = 0..n-1, each held for n_sub sub-steps: xp <- f(xp, clampU(u[j])) with the plant's parameters,
+ * clampU at each sub-step's own state on a fresh copy of u[j] (the reference's forward_pass step; MMex modes 16 then 0), then
+ * x0 <- xp (+ w).  u[j] are the solution's controls, which is also what u_cl logs.  n = 0 leaves x0 (+ w); a host x0 ignores
+ * the plant.  All sub-steps of control j evaluate at step index k = j, and [k]-indexed parameters are the model's (its shared
+ * array, or the window of the solve that just finished).  A non-finite plant state is passed on: the next solve of that problem
+ * fails its initial rollout (result -1), as a host loop would.
+ * Only non-[k]-indexed parameters can be set for the plant (ilqgb_set_param / ilqgb_set_param_batch shapes; batch rows by
+ * global problem index).  An entry never set FOLLOWS THE MODEL: it is, for every problem, the model's current value, shared
+ * or per-problem, including later ilqgb_set_param / ilqgb_set_param_batch calls.  n_sub (1..64) rescales nothing: set the
+ * plant's time-step parameter (h of the car, dt of the quadrotor and the pendulum) to the model's divided by n_sub yourself,
+ * the library does not know which parameter is the time step.  Any of the three setters gives the handle a plant
+ * (ilqgb_set_plant_substeps(h, 1) alone: a plant equal to the model).  ilqgb_clear_plant removes it: x0 <- x[n] (+ w) again,
+ * bit for bit.  ilqgb_get(h, "plant", out) returns the effective plant set of every problem [batch][sum of parameter sizes]
+ * (the "follow the model" rule applied).  Bad index, [k]-indexed parameter, wrong length or n_sub: -1, nothing changed. */
+int ilqgb_set_plant_param(ilqgb_handle *h, int index, const double *value, int n);
+int ilqgb_set_plant_param_batch(ilqgb_handle *h, int index, const double *value, int n);  /* value[batch][n] */
+int ilqgb_set_plant_substeps(ilqgb_handle *h, int n_sub);
+int ilqgb_clear_plant(ilqgb_handle *h);
 
 /* device -> host; any pointer may be NULL. x [batch][n_hor+1][nx], u [batch][n_hor][nu] */
 int ilqgb_download(ilqgb_handle *h, double *x, double *u, double *cost, int *iterations, int *result,
