@@ -109,6 +109,12 @@ int ilqgk_preload(void)
     bad |= preload_one(k_mpc_advance<P>);   /* first launched between two steps of a closed loop, while other chunks solve */
     bad |= preload_one(k_mpc_plant<P, false, false>) | preload_one(k_mpc_plant<P, true, false>);
     if constexpr (HAS_KP) bad |= preload_one(k_mpc_plant<P, false, true>) | preload_one(k_mpc_plant<P, true, true>);
+    bad |= preload_one(k_policy_mark) | preload_one(k_policy_rollout<P, false, false>) | preload_one(k_policy_rollout<P, true, false>);
+    bad |= preload_one(k_policy_eval<P, false, false>) | preload_one(k_policy_eval<P, true, false>);
+    if constexpr (HAS_KP) {
+        bad |= preload_one(k_policy_rollout<P, false, true>) | preload_one(k_policy_rollout<P, true, true>);
+        bad |= preload_one(k_policy_eval<P, false, true>) | preload_one(k_policy_eval<P, true, true>);
+    }
     if (bad) { snprintf(g_err, sizeof g_err, "loading the kernels failed: %s", cudaGetErrorString(cudaGetLastError())); return -1; }
     if (dev >= 0 && dev < ILQGK_MAX_DEVICES) loaded[dev] = 1;
     return 0;
@@ -385,6 +391,35 @@ int ilqgk_launch_mpc_plant(const ilqg_work *w, const ilqg_mpc_step *a, const dou
         else k_mpc_plant<P, false, false><<<grid, 256, 0, (cudaStream_t)stream>>>(*w, *a, pb, *pl);
     }
     return check(cudaGetLastError(), "k_mpc_plant");
+}
+
+int ilqgk_launch_policy_mark(const ilqg_work *w, int *keep, int *policy_ok, int save, void *stream)
+{
+    k_policy_mark<<<nblk(w->B, 256), 256, 0, (cudaStream_t)stream>>>(*w, keep, policy_ok, save);
+    return check(cudaGetLastError(), "k_policy_mark");
+}
+
+int ilqgk_launch_policy_rollout(const ilqg_work *w, const double *params, const ilqg_policy *r, void *stream)
+{
+    /* PER: per-problem parameter table r->pp; TR: [k]-indexed parameters from the tracks */
+    const ParamBlock<P> pb = make_pb(params);
+    const long long lanes = (long long)w->B * r->n_samp;
+    const unsigned grid = (unsigned)((lanes + BP_BLOCK - 1) / BP_BLOCK);
+    if (HAS_KP && w->tr_mask) {
+        constexpr bool TR = HAS_KP;
+        if (r->pp) k_policy_rollout<P, true, TR><<<grid, BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, pb, *r);
+        else k_policy_rollout<P, false, TR><<<grid, BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, pb, *r);
+    } else {
+        if (r->pp) k_policy_rollout<P, true, false><<<grid, BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, pb, *r);
+        else k_policy_rollout<P, false, false><<<grid, BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, pb, *r);
+    }
+    return check(cudaGetLastError(), "k_policy_rollout");
+}
+
+int ilqgk_launch_policy_eval(const ilqg_work *w, const double *params, const int *policy_ok, const double *x, double *u, int k, void *stream)
+{
+    PK_DISPATCH(w, (k_policy_eval<P, PP, TR><<<nblk(w->B, BP_BLOCK), BP_BLOCK, 0, (cudaStream_t)stream>>>(*w, make_pb(params), policy_ok, x, u, k)));
+    return check(cudaGetLastError(), "k_policy_eval");
 }
 
 int ilqgk_launch_scatter(const double *src, double *dst, double *dst_alt, const int *sel, int B, int n_k, int n_i, long long stride_k,

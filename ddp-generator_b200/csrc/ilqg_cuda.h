@@ -66,6 +66,11 @@ int ilqgk_launch_count_active(const ilqg_work *w, int *d_counter, void *stream);
 int ilqgk_launch_mpc_advance(const ilqg_work *w, const ilqg_mpc_step *a, void *stream);
 /* the same with the next state from the plant (k_mpc_plant): params_plant = the shared plant set (used when pl->pp is null) */
 int ilqgk_launch_mpc_plant(const ilqg_work *w, const ilqg_mpc_step *a, const double *params_plant, const ilqg_plant *pl, void *stream);
+/* feedback policy of a solved batch: k_policy_mark (save = 1 before, 0 after the derivative sweep and backward pass of
+   ilqgb_policy), k_policy_rollout (params = the shared set, used when r->pp is null), k_policy_eval (x [B][nx] -> u [B][nu]) */
+int ilqgk_launch_policy_mark(const ilqg_work *w, int *keep /* [7][Bp] */, int *policy_ok, int save, void *stream);
+int ilqgk_launch_policy_rollout(const ilqg_work *w, const double *params, const ilqg_policy *r, void *stream);
+int ilqgk_launch_policy_eval(const ilqg_work *w, const double *params, const int *policy_ok, const double *x, double *u, int k, void *stream);
 /* [B][n_k][n_i] (host order) <-> device element (k, b, i) at base[k*stride_k + b*stride_b + i*stride_i + off] */
 int ilqgk_launch_scatter(const double *src, double *dst, double *dst_alt, const int *sel, int B, int n_k, int n_i, long long stride_k,
                          long long stride_b, long long stride_i, long long off, void *stream);

@@ -49,6 +49,10 @@ struct chunk {
     double *plant_params;       /* [npf] effective shared set (when neither the model nor the plant is per-problem) */
     double *d_plant_eff;        /* [npf][Bp] effective per-problem set, allocated on first use */
     int plant_per;              /* the effective set is d_plant_eff (else plant_params) */
+    /* feedback policy (ilqgb_policy): per problem, whether its gains are valid; what k_policy_mark keeps while the policy's
+       passes run; whether the nominal buffers still hold the gains ilqgb_policy computed (cleared by anything that may move them) */
+    int *d_policy_ok, *d_policy_keep;
+    int policy_valid;
     void *stream;          /* the stream all work of this chunk is enqueued on (stream_main, or stream_io during an end-to-end solve) */
     void *stream_main, *stream_io;
     int owns_stream;
@@ -649,6 +653,9 @@ static chunk *ck_create(int device, int batch, int n_hor, int flags, void *strea
             ilqgk_memset(w->tr_clamp, 0, sizeof(int) * T * Bp, h->stream);
         }
         DALLOC(h->d_counter, int, 1);
+        DALLOC(h->d_policy_ok, int, Bp);
+        DALLOC(h->d_policy_keep, int, 7 * Bp);
+        ilqgk_memset(h->d_policy_ok, 0, sizeof(int) * Bp, h->stream);
     }
     if (ilqgk_host_alloc((void **)&h->h_counter, sizeof(int))) goto oom;
     if (ilqgk_host_alloc((void **)&h->h_poll, sizeof(int) * POLL_RING)) goto oom;
@@ -756,6 +763,7 @@ static int ck_upload(chunk *h, const double *x0, const double *u_nom)
     h->n_launches += 2;
     if (ilqgk_launch_scatter(h->d_stage + B * T * nu, h->w.x0, NULL, NULL, h->B, 1, h->d.nx, 0, 1, h->Bp, 0, h->stream)) return failk(h);
     h->started = 0;
+    h->policy_valid = 0;
     return 0;
 }
 
@@ -783,6 +791,7 @@ static int ck_shift(chunk *h, int n_shift, const double *x0, const double *w)
         h->n_launches++;
     }
     h->started = 0;
+    h->policy_valid = 0;
     return 0;
 }
 
@@ -984,6 +993,7 @@ static int ck_start(chunk *h)
     }
     if (ilqgk_launch_init(&h->w, &h->o, h->params, 7, h->stream)) return failk(h);
     h->n_launches++;
+    h->policy_valid = 0;
     h->iter = 0;
     h->started = 1;
     return 0;
@@ -992,6 +1002,7 @@ static int ck_start(chunk *h)
 static int launch_pass(chunk *h, int do_derivs, int do_back, int do_ls)
 {
     ev_pair *p;
+    h->policy_valid = 0;   /* passes move the trajectories and gains (ck_policy sets it again after its own) */
     if (ensure_traces(h)) return -1;   /* max_iter may have been raised since the solve started */
     if (do_derivs) {
         p = timing_begin(h, TC_DERIVS);
@@ -1083,11 +1094,147 @@ static int ck_phase_backpass_once(chunk *h)
     return rc;
 }
 
+/* ---- feedback policy of a solved batch (see ilqg_b200.h) ---- */
+/* calc_derivs(o); back_pass(o) on every problem: the derivative sweep and one backward pass at the final lambda, through the
+   solver's own launch sequence (ilqgb_phase_derivs + ilqgb_phase_backpass_once); k_policy_mark reaches the finished problems
+   and puts back what that changes */
+static int ck_policy(chunk *h)
+{
+    int rc;
+    if (ilqgk_set_device(h->device)) return failk(h);
+    if (ilqgk_launch_policy_mark(&h->w, h->d_policy_keep, h->d_policy_ok, 1, h->stream)) return failk(h);
+    h->n_launches++;
+    h->o.bp_single = 1;
+    rc = launch_pass(h, 1, 1, 0);
+    h->o.bp_single = 0;
+    if (rc) return -1;
+    if (ilqgk_launch_policy_mark(&h->w, h->d_policy_keep, h->d_policy_ok, 0, h->stream)) return failk(h);
+    h->n_launches++;
+    h->policy_valid = 1;
+    return 0;
+}
+
+/* doubles of the staging buffer one sample of a rollout group needs: x0, cost, final state, ok (as a double), trajectories */
+static size_t policy_sample_doubles(const chunk *h, int traj_x, int traj_u)
+{
+    const size_t nx = (size_t)h->d.nx, nu = (size_t)h->d.nu, T = (size_t)h->T;
+    return 2 * nx + 2 + (traj_x ? (T + 1) * nx : 0) + (traj_u ? T * nu : 0);
+}
+
+/* samples s0 .. s0+g-1 of every problem of the chunk: inputs in, kernel launched.  The group's arrays sit in the staging buffer,
+   [B][g][..] each; a group of all M samples copies straight from the caller's rows, a smaller one is packed on the host. */
+typedef struct {
+    int M, s0, g;
+    const double *x0s;
+    double *cost, *x_final, *x, *u;
+    int *ok;
+} prollout_t;
+
+static void policy_stage_layout(chunk *h, const prollout_t *q, ilqg_policy *r)
+{
+    const size_t Bg = (size_t)h->B * q->g, nx = (size_t)h->d.nx, T = (size_t)h->T;
+    double *s = h->d_stage;
+    r->n_samp = q->g;
+    r->x0s = s;
+    s += Bg * nx;
+    r->cost = s;
+    s += Bg;
+    r->x_final = s;
+    s += Bg * nx;
+    r->ok = (int *)s;
+    s += Bg;
+    r->x = q->x ? s : NULL;
+    s += q->x ? Bg * (T + 1) * nx : 0;
+    r->u = q->u ? s : NULL;
+}
+
+/* copy [B][g][n] between the caller's [B][M][n] rows (from sample s0 on) and a packed host buffer */
+static void policy_pack(const prollout_t *q, int B, size_t n, const double *src, double *dst, int to_packed)
+{
+    int b;
+    for (b = 0; b < B; b++) {
+        const size_t caller = ((size_t)b * q->M + q->s0) * n, packed = (size_t)b * q->g * n;
+        if (to_packed) memcpy(dst + packed, src + caller, sizeof(double) * q->g * n);
+        else memcpy(dst + caller, src + packed, sizeof(double) * q->g * n);
+    }
+}
+
+static int ck_policy_rollout_launch(chunk *h, const prollout_t *q, double *tmp)
+{
+    const size_t Bg = (size_t)h->B * q->g, nx = (size_t)h->d.nx;
+    ilqg_policy r;
+    const double *table = h->params;
+    if (ilqgk_set_device(h->device)) return failk(h);
+    memset(&r, 0, sizeof r);
+    r.pp = h->w.pp;
+    if (h->plant_on) {   /* the plant's effective set: its own entries, the model's elsewhere */
+        if (ck_plant_prepare(h)) return -1;
+        table = h->plant_params;
+        r.pp = h->plant_per ? h->d_plant_eff : NULL;
+    }
+    r.policy_ok = h->d_policy_ok;
+    if (ensure_stage(h, Bg * policy_sample_doubles(h, q->x != NULL, q->u != NULL))) return -1;
+    policy_stage_layout(h, q, &r);
+    if (q->g == q->M) {
+        if (ilqgk_h2d((double *)r.x0s, q->x0s, sizeof(double) * Bg * nx, h->stream)) return failk(h);
+    } else {
+        policy_pack(q, h->B, nx, q->x0s, tmp, 1);
+        if (ilqgk_h2d((double *)r.x0s, tmp, sizeof(double) * Bg * nx, h->stream) || ilqgk_stream_sync(h->stream)) return failk(h);
+    }
+    if (ilqgk_launch_policy_rollout(&h->w, table, &r, h->stream)) return failk(h);
+    h->n_launches++;
+    return 0;
+}
+
+static int ck_policy_rollout_collect(chunk *h, const prollout_t *q, double *tmp)
+{
+    const size_t Bg = (size_t)h->B * q->g, nx = (size_t)h->d.nx, nu = (size_t)h->d.nu, T = (size_t)h->T;
+    ilqg_policy r;
+    if (ilqgk_set_device(h->device)) return failk(h);
+    policy_stage_layout(h, q, &r);
+    if (q->g == q->M) {
+        if (ilqgk_d2h(q->cost, r.cost, sizeof(double) * Bg, h->stream) || ilqgk_d2h(q->x_final, r.x_final, sizeof(double) * Bg * nx, h->stream) ||
+            ilqgk_d2h(q->ok, r.ok, sizeof(int) * Bg, h->stream) || (q->x && ilqgk_d2h(q->x, r.x, sizeof(double) * Bg * (T + 1) * nx, h->stream)) ||
+            (q->u && ilqgk_d2h(q->u, r.u, sizeof(double) * Bg * T * nu, h->stream)))
+            return failk(h);
+        return 0;
+    }
+    {
+        /* a group: through the host buffer, one array at a time */
+        const double *dsrc[4] = {r.cost, r.x_final, r.x, r.u};
+        double *hdst[4] = {q->cost, q->x_final, q->x, q->u};
+        const size_t n[4] = {1, nx, (T + 1) * nx, T * nu};
+        int i, b;
+        for (i = 0; i < 4; i++) {
+            if (!hdst[i]) continue;
+            if (ilqgk_d2h(tmp, dsrc[i], sizeof(double) * Bg * n[i], h->stream) || ilqgk_stream_sync(h->stream)) return failk(h);
+            policy_pack(q, h->B, n[i], tmp, hdst[i], 0);
+        }
+        if (ilqgk_d2h(tmp, r.ok, sizeof(int) * Bg, h->stream) || ilqgk_stream_sync(h->stream)) return failk(h);
+        for (b = 0; b < h->B; b++) memcpy(q->ok + (size_t)b * q->M + q->s0, (const int *)tmp + (size_t)b * q->g, sizeof(int) * q->g);
+    }
+    return 0;
+}
+
+static int ck_policy_eval(chunk *h, int k, const double *x, double *u)
+{
+    const size_t B = (size_t)h->B, nx = (size_t)h->d.nx, nu = (size_t)h->d.nu;
+    if (ilqgk_set_device(h->device)) return failk(h);
+    if (ensure_stage(h, B * (nx + nu))) return -1;
+    if (ilqgk_h2d(h->d_stage, x, sizeof(double) * B * nx, h->stream) ||
+        ilqgk_launch_policy_eval(&h->w, h->params, h->d_policy_ok, h->d_stage, h->d_stage + B * nx, k, h->stream) ||
+        ilqgk_d2h(u, h->d_stage + B * nx, sizeof(double) * B * nu, h->stream) || ilqgk_stream_sync(h->stream))
+        return failk(h);
+    h->n_launches++;
+    return 0;
+}
+
 static int ck_phase_multipliers(chunk *h, int init)
 {
     if (ilqgk_set_device(h->device)) return failk(h);
     if (ilqgk_launch_mult(&h->w, &h->o, h->params, init, h->stream)) return failk(h);
     h->n_launches++;
+    h->policy_valid = 0;
     return 0;
 }
 
@@ -1235,6 +1382,7 @@ static long ck_put(chunk *h, const char *f, const double *in)
     size_t n;
     if (ilqgk_set_device(h->device)) return failk(h);
     if (find_field(h, f, &fd)) return -1;
+    h->policy_valid = 0;
     if (fd.scal) {
         if (ilqgk_h2d(fd.scal, in, sizeof(double) * B, h->stream) || ilqgk_stream_sync(h->stream)) return failk(h);
         return (long)B;
@@ -1267,6 +1415,7 @@ static long ck_get_int(chunk *h, const char *f, int *out)
     else if (!strcmp(f, "n_tails")) scal = w->n_tail;
     else if (!strcmp(f, "bp_done")) scal = w->bp_done;
     else if (!strcmp(f, "deriv_fail")) scal = w->deriv_fail;
+    else if (!strcmp(f, "policy_ok")) scal = h->d_policy_ok;
     {
         /* test hooks: the kernel variant the last backward pass and line search of this chunk ran with.  bp_split: lanes per
            problem of the small-batch backward pass (4) or 0; cw_lpp: lanes per problem of the warp-cooperative backward pass, 0
@@ -1320,6 +1469,7 @@ static long ck_put_int(chunk *h, const char *f, const int *in)
     else if (!strcmp(f, "deriv_fail")) dst = h->w.deriv_fail;
     else if (!strcmp(f, "bp_done")) dst = h->w.bp_done;
     else return fail(h, "unknown field");
+    h->policy_valid = 0;
     if (ilqgk_h2d(dst, in, sizeof(int) * B, h->stream) || ilqgk_stream_sync(h->stream)) return failk(h);
     return (long)B;
 }
@@ -1332,6 +1482,7 @@ static int ck_begin(chunk *h)
     if (ensure_traces(h)) return -1;
     if (ilqgk_launch_init(&h->w, &h->o, h->params, 4, h->stream)) return failk(h);
     h->n_launches++;
+    h->policy_valid = 0;
     h->iter = 0;
     h->started = 1;
     return 0;
@@ -1342,6 +1493,7 @@ static int ck_rollout(chunk *h, double alpha, int cost_only)
     if (ilqgk_set_device(h->device)) return failk(h);
     if (ilqgk_launch_rollout(&h->w, h->params, alpha, cost_only, h->stream)) return failk(h);
     h->n_launches++;
+    h->policy_valid = 0;
     return 0;
 }
 
@@ -1957,6 +2109,89 @@ int ilqgb_clamp_u(ilqgb_handle *h, int k, const double *x, double *u)
     if (ilqgb_sync(h)) return -1;
     for (i = 0; i < h->n; i++)
         if (ck_clamp_u(h->c[i], k, x + (size_t)h->first[i] * h->d.nx, u + (size_t)h->first[i] * h->d.nu)) return hfail(h, h->c[i]);
+    return 0;
+}
+
+/* ---- feedback policy of a solved batch (see ilqg_b200.h) ---- */
+/* staging of one rollout group per chunk: 2^26 doubles (512 MB), so requested trajectories go in groups of samples;
+   ILQG_POLICY_STAGE (doubles) lowers it, which is how the tests reach the grouped path at small sizes */
+#define POLICY_STAGE_DOUBLES ((size_t)1 << 26)
+
+int ilqgb_policy(ilqgb_handle *h)
+{
+    int i;
+    if (fork_streams(h)) return -1;
+    for (i = 0; i < h->n; i++)
+        if (ck_policy(h->c[i])) return hfail(h, h->c[i]);
+    return join_streams(h);
+}
+
+static int policy_ready(ilqgb_handle *h)
+{
+    int i;
+    for (i = 0; i < h->n; i++)
+        if (!h->c[i]->policy_valid) {
+            snprintf(h->err, sizeof h->err, "no current feedback policy: call ilqgb_policy after the solve (an upload, start, begin, shift, "
+                                            "closed loop, solve, pass, rollout or put since then discards it)");
+            return 0;
+        }
+    return 1;
+}
+
+int ilqgb_policy_rollout(ilqgb_handle *h, int M, const double *x0s, double *cost, double *x_final, int *ok, double *x, double *u)
+{
+    const size_t nx = (size_t)h->d.nx, nu = (size_t)h->d.nu, T = (size_t)h->T;
+    size_t G, maxB = 0, per;
+    double *tmp = NULL;
+    int i, s0, rc = 0;
+    if (M < 1) { snprintf(h->err, sizeof h->err, "M must be >= 1"); return -1; }
+    if (!x0s || !cost || !x_final || !ok) { snprintf(h->err, sizeof h->err, "x0s, cost, x_final and ok are required"); return -1; }
+    if (h->c[0]->plant_on && h->c[0]->plant_n_sub > 1) {
+        snprintf(h->err, sizeof h->err, "policy rollouts step the plant once per control: n_sub > 1 is not supported");
+        return -1;
+    }
+    if (!policy_ready(h)) return -1;
+    for (i = 0; i < h->n; i++)
+        if ((size_t)h->c[i]->B > maxB) maxB = (size_t)h->c[i]->B;
+    per = policy_sample_doubles(h->c[0], x != NULL, u != NULL);
+    {
+        const long cap = env_int("ILQG_POLICY_STAGE", 0);
+        G = (cap > 0 && (size_t)cap < POLICY_STAGE_DOUBLES ? (size_t)cap : POLICY_STAGE_DOUBLES) / (maxB * per);
+    }
+    if (G < 1) G = 1;
+    if (G > (size_t)M) G = (size_t)M;
+    if (G < (size_t)M && !(tmp = (double *)malloc(sizeof(double) * maxB * G * per))) { snprintf(h->err, sizeof h->err, "out of host memory"); return -1; }
+    if (fork_streams(h)) { free(tmp); return -1; }
+    for (s0 = 0; s0 < M && !rc; s0 += (int)G) {
+        /* every chunk's group is launched before any is collected, so that the chunks' rollouts run concurrently */
+        for (i = 0; i < h->n && !rc; i++) {
+            const size_t f = (size_t)h->first[i] * M;
+            const prollout_t q = {M, s0, (int)(M - s0 < (int)G ? M - s0 : (int)G), x0s + f * nx, cost + f, x_final + f * nx,
+                                  x ? x + f * (T + 1) * nx : NULL, u ? u + f * T * nu : NULL, ok + f};
+            if (ck_policy_rollout_launch(h->c[i], &q, tmp)) rc = hfail(h, h->c[i]);
+        }
+        for (i = 0; i < h->n && !rc; i++) {
+            const size_t f = (size_t)h->first[i] * M;
+            const prollout_t q = {M, s0, (int)(M - s0 < (int)G ? M - s0 : (int)G), x0s + f * nx, cost + f, x_final + f * nx,
+                                  x ? x + f * (T + 1) * nx : NULL, u ? u + f * T * nu : NULL, ok + f};
+            if (ck_policy_rollout_collect(h->c[i], &q, tmp)) rc = hfail(h, h->c[i]);
+        }
+    }
+    if (join_streams(h)) rc = -1;
+    if (!rc && ilqgb_sync(h)) rc = -1;
+    free(tmp);
+    return rc;
+}
+
+int ilqgb_policy_eval(ilqgb_handle *h, int k, const double *x, double *u)
+{
+    int i;
+    if (k < 0 || k >= h->T) { snprintf(h->err, sizeof h->err, "k must be in 0..n_hor-1"); return -1; }
+    if (!x || !u) { snprintf(h->err, sizeof h->err, "x and u are required"); return -1; }
+    if (!policy_ready(h)) return -1;
+    if (ilqgb_sync(h)) return -1;
+    for (i = 0; i < h->n; i++)
+        if (ck_policy_eval(h->c[i], k, x + (size_t)h->first[i] * h->d.nx, u + (size_t)h->first[i] * h->d.nu)) return hfail(h, h->c[i]);
     return 0;
 }
 

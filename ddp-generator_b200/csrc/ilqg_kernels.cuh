@@ -2240,6 +2240,179 @@ __global__ void __launch_bounds__(256) k_mpc_plant(Work w, ilqg_mpc_step a, Para
     mpc_log_shift<P>(w, a, b, src, xn);
 }
 
+/* =====================================================================================================================
+ * Feedback policy of a solved batch (ilqgb_policy, ilqgb_policy_rollout, ilqgb_policy_eval).
+ * ===================================================================================================================== */
+/* ilqgb_policy runs the derivative sweep and one backward pass on every problem, finished or not.  save = 1 (before): keep what
+   reaching finished problems changes -- status, new_deriv, deriv_fail, and the iterations / result / counters that the backward
+   pass's derivative-failure exit and bookkeeping write -- then mark every problem running with fresh derivatives and no
+   successful backward pass.  save = 0 (after): policy_ok = finite derivatives and a successful backward pass; restore. */
+__global__ void k_policy_mark(Work w, int *keep /* [7][Bp] */, int *policy_ok, int save)
+{
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= w.B) return;
+    const size_t Bp = w.Bp;
+    if (save) {
+        keep[0 * Bp + b] = w.status[b];
+        keep[1 * Bp + b] = w.new_deriv[b];
+        keep[2 * Bp + b] = w.deriv_fail[b];
+        keep[3 * Bp + b] = w.iterations[b];
+        keep[4 * Bp + b] = w.result[b];
+        keep[5 * Bp + b] = w.n_bp[b];
+        keep[6 * Bp + b] = w.n_dv[b];
+        w.status[b] = ST_RUNNING;
+        w.new_deriv[b] = 1;
+        w.deriv_fail[b] = 0;
+        w.bp_done[b] = 0;
+    } else {
+        policy_ok[b] = (!w.deriv_fail[b] && w.bp_done[b]) ? 1 : 0;
+        w.status[b] = keep[0 * Bp + b];
+        w.new_deriv[b] = keep[1 * Bp + b];
+        w.deriv_fail[b] = keep[2 * Bp + b];
+        w.iterations[b] = keep[3 * Bp + b];
+        w.result[b] = keep[4 * Bp + b];
+        w.n_bp[b] = keep[5 * Bp + b];
+        w.n_dv[b] = keep[6 * Bp + b];
+    }
+}
+
+/* u_k(x) = u*_k + 0 * l_k + L_k (x - x*_k): the feedback expression of forward_pass (iLQG_func.tem:121-185) at alpha = 0, in its
+   order of operations.  (forward_pass itself takes the open-loop branch when alpha == 0.)  The 0 * l term stays: it decides the
+   sign of a zero control.  nom = x* | u* of step k, ll = l | L of step k. */
+template <class P>
+__device__ __forceinline__ void policy_u(const double *nom, const double *ll, const double *x, double *u)
+{
+    constexpr int NX = P::NX, NU = P::NU;
+#pragma unroll
+    for (int j = 0; j < NU; j++) u[j] = nom[NX + j] + ll[j] * 0.0;
+#pragma unroll
+    for (int i = 0; i < NX; i++) {
+        const double dx = x[i] - nom[i];
+#pragma unroll
+        for (int j = 0; j < NU; j++) u[j] += ll[NU + j + i * NU] * dx;
+    }
+}
+
+/* the nominal x|u, l and L records of step k of problem b, from the nominal buffer, whose gains ilqgb_policy wrote */
+template <class P>
+__device__ __forceinline__ void policy_records(const Work &w, int b, int cur, int k, double *nom, double *ll)
+{
+    const size_t i = (size_t)k * w.Bp + b;
+    ld_rec<P::NX + P::NU>(w.XU[cur] + i * Rec<P>::RXU, nom);
+    ld_rec<P::NU>(w.Ll[cur] + i * Rec<P>::RLS, ll);
+    ld_rec<P::NU * P::NX>(w.LL[cur] + i * Rec<P>::RLM, ll + P::NU);
+}
+
+/* Closed-loop rollouts of the feedback policy, one lane per (problem b, sample s), lane b * n_samp + s: forward_pass(candidate, o,
+ * 0, &csum, 0) with the gains applied (policy_u), from x0s[b][s], with the final multipliers and penalty weights, clampU at the
+ * rollout's own state and, where the handle has a plant, the plant's parameters for the whole step (clampU, f and cost).  The
+ * samples of a problem sit in adjacent lanes: a warp reads each nominal record once and broadcasts it to them (one problem per
+ * warp from n_samp = 32 on), so the nominal traffic per step is that of one rollout per problem whatever n_samp is.  Nothing is
+ * written to the handle's trajectory buffers; x / u rows are stored only when asked for.  A problem without a valid policy, and a
+ * rollout that fails, give ok = 0, NaN cost and NaN final state; the stored rows of a failed rollout end with the failing step
+ * and the rest are NaN.  PER: parameters from r.pp ([NPF][Bp]); TR: [k]-indexed parameters from the tracks' window. */
+template <class P, bool PER, bool TR = false>
+__global__ void __launch_bounds__(BP_BLOCK, ILQG_LS_MINBLOCKS) k_policy_rollout(Work w, ParamBlock<P> pb, ilqg_policy r)
+{
+    constexpr int NX = P::NX, NU = P::NU, RLM = Rec<P>::RLM;
+    const size_t row = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int b = (int)(row / (size_t)r.n_samp);
+    if (b >= w.B) return;
+    const size_t Bp = w.Bp;
+    const int T = w.T;
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    double x[NX], xn[NX], u[NU], mu[P::N_MU_R + P::N_MU_F + 1], nom[Rec<P>::RXU], ll[NU + RLM];
+#pragma unroll
+    for (int i = 0; i < NX; i++) x[i] = r.x0s[row * NX + i];
+    double *xs = r.x ? r.x + row * (size_t)(T + 1) * NX : nullptr;
+    double *us = r.u ? r.u + row * (size_t)T * NU : nullptr;
+    bool ok = r.policy_ok[b] != 0;
+    double csum = 0.0;
+    int stored = 0;   /* x / u rows written */
+    if (ok) {
+        double pl_[PER ? P::NPF : 1];
+        const double *pv = pb.v;
+        if (PER) {
+#pragma unroll
+            for (int i = 0; i < P::NPF_USED; i++) pl_[i] = r.pp[(size_t)i * Bp + b];
+            pv = pl_;
+        }
+        ILQG_PK(TR, b)
+        const int cur = w.cur[b];
+        const double w_pen_l = w.w_pen_l[b];
+        for (int k = 0; k < T; k++) {
+            policy_records<P>(w, b, cur, k, nom, ll);
+            policy_u<P>(nom, ll, x, u);
+#pragma unroll
+            for (int i = 0; i < P::N_MU_R; i++) mu[i] = w.muR[((size_t)k * P::N_MU_R + i) * Bp + b];
+            double c;
+            ok = P::step(x, u, pv, pk, k, T, w_pen_l, mu, xn, c);
+            if (xs) {
+#pragma unroll
+                for (int i = 0; i < NX; i++) xs[(size_t)k * NX + i] = x[i];
+            }
+            if (us) {
+#pragma unroll
+                for (int j = 0; j < NU; j++) us[(size_t)k * NU + j] = u[j];
+            }
+            stored = k + 1;
+            if (!ok) break;
+            csum += c;
+#pragma unroll
+            for (int i = 0; i < NX; i++) x[i] = xn[i];
+        }
+        if (ok) {
+#pragma unroll
+            for (int i = 0; i < P::N_MU_F; i++) mu[i] = w.muF[(size_t)i * Bp + b];
+            double c;
+            ok = P::final_cost(x, pv, pk, T, T, w.w_pen_f[b], mu, c);
+            csum += c;
+            if (ok && xs) {
+#pragma unroll
+                for (int i = 0; i < NX; i++) xs[(size_t)T * NX + i] = x[i];
+            }
+        }
+    }
+    r.ok[row] = ok ? 1 : 0;
+    r.cost[row] = ok ? csum : nan;
+#pragma unroll
+    for (int i = 0; i < NX; i++) r.x_final[row * NX + i] = ok ? x[i] : nan;
+    if (!ok) {
+        if (xs)
+            for (size_t i = (size_t)stored * NX; i < (size_t)(T + 1) * NX; i++) xs[i] = nan;
+        if (us)
+            for (size_t i = (size_t)stored * NU; i < (size_t)T * NU; i++) us[i] = nan;
+    }
+}
+
+/* The policy's control at step k for one state per problem (ilqgb_policy_eval): step k of k_policy_rollout without f, with the
+   model's parameters -- policy_u, then clampU at x as in k_clamp.  x [B][NX] in, u [B][NU] out; NaN without a valid policy. */
+template <class P, bool PP, bool TR = false>
+__global__ void __launch_bounds__(BP_BLOCK) k_policy_eval(Work w, ParamBlock<P> pb, const int *policy_ok, const double *xin, double *uout, int k)
+{
+    constexpr int NX = P::NX, NU = P::NU;
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= w.B) return;
+    double *uo = uout + (size_t)b * NU;
+    if (!policy_ok[b]) {
+#pragma unroll
+        for (int j = 0; j < NU; j++) uo[j] = __longlong_as_double(0x7ff8000000000000LL);
+        return;
+    }
+    ILQG_PARAMS(PP, b)
+    ILQG_PK(TR, b)
+    double x[NX], xn[NX], u[NU], mu[P::N_MU_R + P::N_MU_F + 1], nom[Rec<P>::RXU], ll[NU + Rec<P>::RLM], c;
+#pragma unroll
+    for (int i = 0; i < NX; i++) x[i] = xin[(size_t)b * NX + i];
+    policy_records<P>(w, b, w.cur[b], k, nom, ll);
+    policy_u<P>(nom, ll, x, u);
+#pragma unroll
+    for (int i = 0; i < P::N_MU_R; i++) mu[i] = 0.0;
+    P::step(x, u, pv, pk, k, w.T, 0.0, mu, xn, c);   /* the clamp is the first thing a step does to u */
+#pragma unroll
+    for (int j = 0; j < NU; j++) uo[j] = u[j];
+}
+
 /* layout changes between the caller's problem-major arrays [B][n_k][n_i] and device arrays addressed as
  * base[(k * stride_k + b) * stride_b + off + i * stride_i]  (records: stride_k = Bp, stride_b = record size, stride_i = 1;
  * structure-of-arrays [k][i][Bp]: handled by the caller passing stride_b = 1, stride_i = Bp, stride_k = n_i * Bp / 1) */

@@ -75,4 +75,17 @@ typedef struct ilqg_plant {
     const double *pp;   /* per-problem plant parameter sets [NPF][Bp], or null = one shared set (kernel argument) */
 } ilqg_plant;
 
+/* one launch of k_policy_rollout: n_samp closed-loop rollouts of the feedback policy per problem, lane b * n_samp + s.  The
+ * arrays are problem-major ([B][n_samp][..]) so that they copy to and from the caller's arrays without a layout change.  Like
+ * ilqg_plant it travels in the kernel's own arguments. */
+typedef struct ilqg_policy {
+    int n_samp;             /* samples per problem in this launch */
+    const int *policy_ok;   /* [Bp] the problem's gains are valid (ilqgb_policy) */
+    const double *pp;       /* per-problem parameter sets [NPF][Bp] (the model's or the plant's), or null = one shared set */
+    const double *x0s;      /* [B][n_samp][NX] initial states */
+    double *cost, *x_final; /* [B][n_samp], [B][n_samp][NX] */
+    int *ok;                /* [B][n_samp] forward_pass's return value */
+    double *x, *u;          /* [B][n_samp][T+1][NX], [B][n_samp][T][NU], or null = not stored */
+} ilqg_policy;
+
 #endif

@@ -22,7 +22,7 @@ TRACE, TIMING = 1, 2
 KERNEL_CLASSES = ("derivs", "backpass", "linesearch", "post")
 _SCALAR_FIELDS = {"cost", "new_cost", "dcost", "expected", "lambda", "dlambda", "g_norm", "dV0", "dV1", "w_pen_l", "w_pen_f",
                   "iterations", "result", "status", "n_linesearch", "n_backpass", "n_derivs", "n_rollouts", "n_tails", "cur", "bp_split",
-                  "cw_lpp", "bp_latency", "ls_tail_from", "ls_commit_par"}
+                  "cw_lpp", "bp_latency", "ls_tail_from", "ls_commit_par", "policy_ok"}
 
 
 def lib_path(problem, full_ddp, lib_dir=None):
@@ -97,6 +97,9 @@ class Library:
         L.ilqgb_launch_count.argtypes = [vp]
         L.ilqgb_chunks.argtypes = [vp]
         L.ilqgb_set_tuning.argtypes = [vp, cp, ci]
+        L.ilqgb_policy.argtypes = [vp]
+        L.ilqgb_policy_rollout.argtypes = [vp, ci, dp, dp, dp, dp, dp, dp]
+        L.ilqgb_policy_eval.argtypes = [vp, ci, dp, dp]
         self.problem = L.ilqgb_problem_name().decode()
         self.nx, self.nu = L.ilqgb_nx(), L.ilqgb_nu()
         self.full_ddp = L.ilqgb_full_ddp()
@@ -323,6 +326,35 @@ class BatchSolver:
                    iterations=np.empty((self.B, S), np.int32), success=np.empty((self.B, S), np.int32))
         self._chk(self.lib.ilqgb_mpc(self.h, S, _ptr(x0), _ptr(u0), _ptr(w), *[_ptr(out[k]) for k in ("x", "u", "cost", "iterations", "success")]))
         return out
+
+    # feedback policy of a solved batch ------------------------------------------------------------------------------------
+    def policy(self):
+        """Gains at the final trajectory of every problem (ilqgb_policy): calc_derivs + one back_pass at the final lambda.
+        get_int("policy_ok") says which problems got them.  Valid until the next upload, start, shift, mpc, solve or put."""
+        self._chk(self.lib.ilqgb_policy(self.h))
+
+    def policy_rollout(self, x0s, want_traj=False):
+        """Closed-loop rollouts of the policy from x0s [B, M, nx] (ilqgb_policy_rollout): u = u*_k + L_k (x - x*_k), clamped, then
+        the model's (or the plant's) dynamics.  Returns cost [B, M], x_final [B, M, nx], ok [B, M] and, with want_traj,
+        x [B, M, T+1, nx] and u [B, M, T, nu].  The handle is left as it was."""
+        x0s = np.ascontiguousarray(x0s, dtype=np.float64)
+        if x0s.ndim != 3 or x0s.shape[0] != self.B or x0s.shape[2] != self.nx:
+            raise ValueError(f"x0s must be [batch, M, nx] = [{self.B}, M, {self.nx}], got {list(x0s.shape)}")
+        B, M = self.B, x0s.shape[1]
+        out = dict(cost=np.empty((B, M)), x_final=np.empty((B, M, self.nx)), ok=np.empty((B, M), np.int32))
+        if want_traj:
+            out["x"] = np.empty((B, M, self.T + 1, self.nx))
+            out["u"] = np.empty((B, M, self.T, self.nu))
+        self._chk(self.lib.ilqgb_policy_rollout(self.h, M, _ptr(x0s), _ptr(out["cost"]), _ptr(out["x_final"]), _ptr(out["ok"]),
+                                                _ptr(out.get("x")), _ptr(out.get("u"))))
+        return out
+
+    def policy_eval(self, k, x):
+        """The policy's control at step k for one state per problem, x [B, nx] -> u [B, nu] (ilqgb_policy_eval)."""
+        x = self._state("x", x, (self.B, self.nx))
+        u = np.empty((self.B, self.nu))
+        self._chk(self.lib.ilqgb_policy_eval(self.h, int(k), _ptr(x), _ptr(u)))
+        return u
 
     def set_tuning(self, name, value):
         """Run-time tuning knobs (ilqgb_set_tuning): ls_tail_from, bp_latency, bp_split, cw_lpp, pass_index."""

@@ -42,6 +42,17 @@ def disturbance(B, S, nx, scale, seed, first=0):
     return scale * normal(seed, b[:, None], idx).reshape(B, S, nx)
 
 
+def perturbed_states(x0, M, scale, seed, first=0):
+    """M initial states per problem around x0 [B, nx] for Monte-Carlo rollouts of a feedback policy (BatchSolver.policy_rollout):
+    x0s [B, M, nx] = x0[b] + scale * N(0,1), scale a scalar or one value per state; rows are problems first..first+B-1, so a
+    shard regenerates its own."""
+    x0 = np.asarray(x0, dtype=np.float64)
+    B, nx = x0.shape
+    b = np.arange(first, first + B, dtype=np.uint64)
+    idx = np.arange(M * nx, dtype=np.uint64)[None, :]
+    return x0[:, None, :] + np.asarray(scale, dtype=np.float64) * normal(seed, b[:, None], idx).reshape(B, M, nx)
+
+
 def _scaled(seed, b, idx, nominal, spread):
     """nominal values scaled by U(1 - spread, 1 + spread), one factor per problem b and element idx"""
     return np.asarray(nominal)[None, :] * (1.0 + spread * (2.0 * uniform01(seed, b[:, None], idx[None, :]) - 1.0))

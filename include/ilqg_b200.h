@@ -22,6 +22,8 @@
  *                                  previous u, shifted, is the next u_nom), on the device; ilqgb_mpc runs whole closed loops
  *   ilqgb_set_plant_*              the plant of such a loop, which the caller steps with iLQG<Name>MMex modes 16 and 0 and
  *                                  the plant's parameter struct (iLQG_MMex.tem:81-226)
+ *   ilqgb_policy / _policy_rollout calc_derivs + back_pass on the tOptSet iLQG() left behind, then forward_pass's feedback step
+ *   / _policy_eval                 from other initial states: the solved controller's local feedback law, rolled out on the device
  *   ilqgb_phase_*                  calc_derivs / back_pass / line_search on their own (iLQG.h:83, back_pass.h:7,
  *                                  line_search.h:6) for phase-level parity tests
  *   ilqgb_get / ilqgb_get_int      read-back of any per-problem field (tOptSet / trajEl_t members)
@@ -140,6 +142,31 @@ int ilqgb_set_plant_param(ilqgb_handle *h, int index, const double *value, int n
 int ilqgb_set_plant_param_batch(ilqgb_handle *h, int index, const double *value, int n);  /* value[batch][n] */
 int ilqgb_set_plant_substeps(ilqgb_handle *h, int n_sub);
 int ilqgb_clear_plant(ilqgb_handle *h);
+
+/* Feedback policy of a solved batch.  A solve leaves a plan (x*, u*) and a local feedback law u_k(x) = u*_k + L_k (x - x*_k).
+ * ilqgb_policy computes the gains at the final trajectory: for every problem, finished or not, exactly calc_derivs(o); back_pass(o)
+ * on the tOptSet iLQG(o) left behind (iLQG.h:83, back_pass.h:7) -- one derivative sweep and ONE backward pass at the final lambda,
+ * with the final multipliers and penalty weights, no regularisation retry, no gradient exit.  Afterwards "l" "L" "dV0" "dV1"
+ * "g_norm" "v1" "v2" "fd" and "bp_done" hold what back_pass writes; x, u, cost, iterations, result, status, lambda, dlambda, cur
+ * and the multipliers are unchanged.  ilqgb_get_int(h, "policy_ok") = derivatives finite and backward pass successful
+ * (bp_done).  Asynchronous.  The policy stays valid until the next ilqgb_upload, _start, _begin, _shift, _mpc, _solve*,
+ * _iterate, _phase_*, _rollout or ilqgb_put*; after those ilqgb_policy_rollout and ilqgb_policy_eval fail. */
+int ilqgb_policy(ilqgb_handle *h);
+/* M >= 1 closed-loop rollouts of the policy per problem from x0s [batch][M][nx]: sample (b, i) is forward_pass(candidate, o, alpha,
+ * &csum, 0) (iLQG_func.tem:121-185) with alpha's feedback branch taken at alpha = 0 -- u = u*_k + 0 * l_k + L_k (x - x*_k), then
+ * clampU at the rollout's own state, then f -- from o.x0 = x0s[b][i].  (forward_pass skips the gains when alpha == 0 exactly;
+ * a rollout here always applies them.)  With a plant (ilqgb_set_plant_*), o.p is problem b's effective plant set (ilqgb_get
+ * "plant") for the whole step; otherwise the model's.  [k]-indexed parameters: the model's, through the solve's track window.
+ * cost [batch][M] = csum (running and final cost with the final multipliers and penalty weights), ok [batch][M] = forward_pass's
+ * return value, x_final [batch][M][nx]; x [batch][M][n_hor+1][nx] and u [batch][M][n_hor][nu] (the clamped controls) are
+ * optional (NULL).  A problem with policy_ok == 0, and a rollout that fails, give ok = 0 and NaN cost and final state (logged rows
+ * after the failing step: NaN).  Nothing of the handle changes: its trajectories, download and get stay as they were.  Needs
+ * ilqgb_policy since the last solve; plant sub-steps (n_sub > 1) are rejected.  Rows by global problem index.  Synchronises. */
+int ilqgb_policy_rollout(ilqgb_handle *h, int M, const double *x0s, double *cost, double *x_final, int *ok, double *x, double *u);
+/* the policy's control at step k (0 <= k < n_hor) for one state per problem, x [batch][nx] -> u [batch][nu]: step k of a policy
+ * rollout without f, with the model's parameters (the controller's own limits).  NaN for problems with policy_ok == 0.  For
+ * callers that step their own simulator.  Synchronises. */
+int ilqgb_policy_eval(ilqgb_handle *h, int k, const double *x, double *u);
 
 /* device -> host; any pointer may be NULL. x [batch][n_hor+1][nx], u [batch][n_hor][nu] */
 int ilqgb_download(ilqgb_handle *h, double *x, double *u, double *cost, int *iterations, int *result,
