@@ -93,6 +93,40 @@ template <bool PP> static int preload_pp()
 
 constexpr bool HAS_KP = P::NKP > 0;
 
+static inline unsigned nblk(int n, int bs) { return (unsigned)((n + bs - 1) / bs); }
+
+/* k_backpass_warp at LPP lanes per problem.  The opt-in to more than 48 KB of dynamic shared memory is a per-device function
+   attribute, set for the variant launched only: at 8 lanes per problem the workspace of a large problem can exceed what the device
+   gives a block while 32 lanes fit (the handle rejects such a setting, ilqgk_coop_smem) */
+template <int LPP> static int cw_launch(const ilqg_work *w, const ilqg_opts *o, const double *params, int iter, void *stream)
+{
+    constexpr bool FULL = FULL_DDP != 0;
+    constexpr int smem = (int)coop_smem_bytes<P, LPP>();
+    static unsigned char configured[ILQGK_MAX_DEVICES];
+    int dev = 0;
+    if (check(cudaGetDevice(&dev), "cudaGetDevice")) return -1;
+    if (dev < 0 || dev >= ILQGK_MAX_DEVICES || !configured[dev]) {
+        if (check(cudaFuncSetAttribute(k_backpass_warp<P, FULL, false, LPP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem), "cudaFuncSetAttribute") ||
+            check(cudaFuncSetAttribute(k_backpass_warp<P, FULL, true, LPP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem), "cudaFuncSetAttribute"))
+            return -1;
+        if (dev >= 0 && dev < ILQGK_MAX_DEVICES) configured[dev] = 1;
+    }
+    const unsigned grid = nblk(w->B, CW_WARPS * (32 / LPP));
+    if (w->pp) k_backpass_warp<P, FULL, true, LPP><<<grid, CW_WARPS * 32, smem, (cudaStream_t)stream>>>(*w, *o, make_pb(params), iter);
+    else k_backpass_warp<P, FULL, false, LPP><<<grid, CW_WARPS * 32, smem, (cudaStream_t)stream>>>(*w, *o, make_pb(params), iter);
+    return check(cudaGetLastError(), "k_backpass");
+}
+
+template <int LPP> static int cw_smem(size_t *need)
+{
+    cudaFuncAttributes a, b;
+    if (check(cudaFuncGetAttributes(&a, k_backpass_warp<P, FULL_DDP != 0, false, LPP>), "cudaFuncGetAttributes") ||
+        check(cudaFuncGetAttributes(&b, k_backpass_warp<P, FULL_DDP != 0, true, LPP>), "cudaFuncGetAttributes"))
+        return -1;
+    *need = coop_smem_bytes<P, LPP>() + (a.sharedSizeBytes > b.sharedSizeBytes ? a.sharedSizeBytes : b.sharedSizeBytes);
+    return 0;
+}
+
 extern "C" {
 
 const char *ilqgk_last_error(void) { return g_err; }
@@ -133,6 +167,21 @@ const char *ilqgk_problem_name(void) { return P::name(); }
 int ilqgk_param_count(void) { return P::param_count(); }
 const char *ilqgk_param_name(int i) { return P::param_name(i); }
 int ilqgk_param_size(int i) { return P::param_size(i); }
+
+int ilqgk_coop_smem(int dev, int lpp, size_t *need, size_t *limit)
+{
+    /* queried on device `dev`; the calling thread's current device is restored */
+    int prev = 0, optin = 0, rc = 0;
+    *need = *limit = 0;
+    if constexpr (use_coop<P>()) {
+        if (check(cudaGetDevice(&prev), "cudaGetDevice") || check(cudaSetDevice(dev), "cudaSetDevice")) return -1;
+        rc = check(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev), "cudaDeviceGetAttribute");
+        if (!rc) rc = lpp == 8 ? cw_smem<8>(need) : lpp == 16 ? cw_smem<16>(need) : cw_smem<32>(need);
+        *limit = (size_t)optin;
+        if (check(cudaSetDevice(prev), "cudaSetDevice")) return -1;
+    }
+    return rc;
+}
 
 int ilqgk_device_count(void) { int n = 0; if (cudaGetDeviceCount(&n) != cudaSuccess) return 0; return n; }
 int ilqgk_set_device(int dev) { return check(cudaSetDevice(dev), "cudaSetDevice"); }
@@ -177,8 +226,6 @@ int ilqgk_event_destroy(void *e) { return check(cudaEventDestroy((cudaEvent_t)e)
 int ilqgk_event_record(void *e, void *s) { return check(cudaEventRecord((cudaEvent_t)e, (cudaStream_t)s), "cudaEventRecord"); }
 int ilqgk_event_elapsed(void *a, void *b, float *ms) { return check(cudaEventElapsedTime(ms, (cudaEvent_t)a, (cudaEvent_t)b), "cudaEventElapsedTime"); }
 
-static inline unsigned nblk(int n, int bs) { return (unsigned)((n + bs - 1) / bs); }
-
 /* every solver kernel exists for shared parameters and for per-problem parameter sets */
 #define PP_DISPATCH(w_, CALL)          \
     do {                               \
@@ -215,20 +262,9 @@ int ilqgk_launch_backpass(const ilqg_work *w, const ilqg_opts *o, const double *
 {
     if constexpr (use_coop<P>()) {
         /* lanes per problem: 32, 16 or 8 (o->cw_lpp); the workspace of all problems of a block sits in dynamic shared memory */
-        static unsigned char cw_configured[ILQGK_MAX_DEVICES];
-        int dev = 0;
-        if (check(cudaGetDevice(&dev), "cudaGetDevice")) return -1;
-#define CW_ATTR(LPP_, PP_) check(cudaFuncSetAttribute(k_backpass_warp<P, FULL_DDP != 0, PP_, LPP_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coop_smem_bytes<P, LPP_>()), "cudaFuncSetAttribute")
-        if (dev < 0 || dev >= ILQGK_MAX_DEVICES || !cw_configured[dev]) {
-            if (CW_ATTR(32, false) || CW_ATTR(32, true) || CW_ATTR(16, false) || CW_ATTR(16, true) || CW_ATTR(8, false) || CW_ATTR(8, true)) return -1;
-            if (dev >= 0 && dev < ILQGK_MAX_DEVICES) cw_configured[dev] = 1;
-        }
-#undef CW_ATTR
-#define CW_LAUNCH(LPP_) PP_DISPATCH(w, (k_backpass_warp<P, FULL_DDP != 0, PP, LPP_><<<nblk(w->B, CW_WARPS * (32 / LPP_)), CW_WARPS * 32, coop_smem_bytes<P, LPP_>(), (cudaStream_t)stream>>>(*w, *o, make_pb(params), iter)))
-        if (o->cw_lpp == 8) CW_LAUNCH(8);
-        else if (o->cw_lpp == 16) CW_LAUNCH(16);
-        else CW_LAUNCH(32);
-#undef CW_LAUNCH
+        if (o->cw_lpp == 8) return cw_launch<8>(w, o, params, iter, stream);
+        if (o->cw_lpp == 16) return cw_launch<16>(w, o, params, iter, stream);
+        return cw_launch<32>(w, o, params, iter, stream);
     }
     else {
         constexpr size_t smem = sizeof(double) * 2 * bp_fields<P, FULL_DDP != 0>() * BP_BLOCK;

@@ -20,6 +20,9 @@ const char *ilqgk_param_name(int i);
 int ilqgk_param_size(int i);
 
 int ilqgk_preload(void); /* load every solver kernel on the current device (idempotent) */
+/* shared memory one block of the warp-cooperative backward pass needs at lpp lanes per problem, and what device dev gives a block
+   after opt-in (both 0 where the problem does not use that kernel); leaves the calling thread's current device as it was */
+int ilqgk_coop_smem(int dev, int lpp, size_t *need, size_t *limit);
 int ilqgk_device_count(void);
 int ilqgk_set_device(int dev);
 int ilqgk_malloc(void **p, size_t bytes);

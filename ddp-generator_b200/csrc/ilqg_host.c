@@ -110,6 +110,21 @@ static int env_int(const char *name, int dflt)
     return v && *v ? atoi(v) : dflt;
 }
 
+/* The warp-cooperative backward pass keeps the workspace of every problem of a block in shared memory, 32 / lpp problems per warp:
+   a lanes-per-problem count whose workspace the device cannot give a block is refused here, not in the middle of a solve */
+static int coop_fits(const chunk *h, int lpp, char *err, size_t n)
+{
+    size_t need = 0, limit = 0;
+    if (!h->d.coop) return 1;
+    if (ilqgk_coop_smem(h->device, lpp, &need, &limit)) {
+        snprintf(err, n, "%s", ilqgk_last_error());
+        return 0;
+    }
+    if (need <= limit) return 1;
+    snprintf(err, n, "cw_lpp %d: the warp-cooperative backward pass needs %zu bytes of shared memory per block, the device allows %zu", lpp, need, limit);
+    return 0;
+}
+
 static void *dalloc(chunk *h, size_t bytes)
 {
     void *p = NULL;
@@ -549,6 +564,10 @@ static chunk *ck_create(int device, int batch, int n_hor, int flags, void *strea
     }
     if (h->d.nkp > 16) {
         fail(NULL, "too many [k]-indexed parameters");
+        free(h);
+        return NULL;
+    }
+    if (!coop_fits(h, 32, g_create_err, sizeof g_create_err) || !coop_fits(h, h->cw_lpp, g_create_err, sizeof g_create_err)) {
         free(h);
         return NULL;
     }
@@ -2226,6 +2245,9 @@ int ilqgb_eval(ilqgb_handle *h, int mode, int k, const double *x, const double *
 int ilqgb_set_tuning(ilqgb_handle *h, const char *name, int value)
 {
     int i;
+    if (!strcmp(name, "cw_lpp"))
+        for (i = 0; i < h->n; i++)
+            if ((value == 32 || value == 16 || value == 8) && !coop_fits(h->c[i], value, h->err, sizeof h->err)) return -1;
     for (i = 0; i < h->n; i++) {
         if (!strcmp(name, "ls_tail_from")) h->c[i]->ls_tail_from = value;
         else if (!strcmp(name, "pass_index")) { h->c[i]->iter = value; h->c[i]->started = 1; }

@@ -204,7 +204,8 @@ int ilqgb_dense_size(void);
 /* run-time tuning knobs, otherwise chosen from the batch size: "ls_tail_from" (sequential line-search rounds before the
  * parallel-alpha tail; >= n_alpha: all rounds sequential, every tried rollout is stored as in the reference), "bp_latency";
  * "bp_split": lanes per problem of the backward pass, 4 = the small-batch kernel k_backpass_split (problems without state-dependent input
- * limits; ignored otherwise), 0 = one lane per problem, -1 = by batch size; "cw_lpp";
+ * limits; ignored otherwise), 0 = one lane per problem, -1 = by batch size; "cw_lpp" (32, 16 or 8; refused, and the handle
+ * unchanged, when the workspace of 32 / value problems per warp does not fit in a block's shared memory: the error names the bytes);
  * "pass_index": the loop index the next ilqgb_phase_* call runs as (row of the traces) */
 int ilqgb_set_tuning(ilqgb_handle *h, const char *name, int value);
 

@@ -17,15 +17,16 @@ ROOT = oracle_lib.ROOT
 _SHIMS = {}
 
 
-def shim(problem, ddp):
-    """tests/policy_oracle_shim.c compiled against the problem's structure layout, as the oracle's own C is (oracle/Makefile)"""
+def shim(problem, ddp, probdir=None):
+    """tests/policy_oracle_shim.c compiled against the problem's structure layout, as the oracle's own C is (oracle/Makefile);
+    `probdir`: the root of the generated problem code where it is not the package's problems/"""
     key = (problem, int(ddp))
     if key not in _SHIMS:
         out = os.path.join(tempfile.mkdtemp(prefix="policy_shim_"), f"shim_{problem}_{int(ddp)}.so")
         subprocess.run(["gcc", "-O2", "-ffp-contract=off", "-fPIC", "-shared", "-std=gnu11", "-w", "-DHAVE_OCTAVE", "-DPRNT=h_prnt",
                         f"-DFULL_DDP={int(ddp)}", "-include", os.path.join(ROOT, "oracle", "prnt_decl.h"),
                         "-I" + os.path.join(ROOT, "oracle", "mex_stub"), "-I" + os.path.join(ROOT, "ddp-generator_b200", "csrc"),
-                        "-I" + os.path.join(ROOT, "ddp-generator_b200", "problems", problem), "-I" + os.path.join(ROOT, "include"),
+                        "-I" + os.path.join(probdir or os.path.join(ROOT, "ddp-generator_b200", "problems"), problem), "-I" + os.path.join(ROOT, "include"),
                         os.path.join(ROOT, "tests", "policy_oracle_shim.c"), "-o", out], check=True)
         L = C.CDLL(out)
         L.ps_set_x0.argtypes = [C.c_void_p, oracle_lib._dp]
@@ -34,9 +35,9 @@ def shim(problem, ddp):
     return _SHIMS[key]
 
 
-def oracle(problem, ddp):
+def oracle(problem, ddp, probdir=None):
     O = oracle_lib.OracleLib(PU.oracle_kinds(problem, ddp)[0], problem, ddp)
-    O.shim = shim(problem, ddp)
+    O.shim = shim(problem, ddp, probdir)
     return O
 
 

@@ -12,12 +12,13 @@ import pytest
 
 import fake_mex as FM
 import oracle_lib
+import shapes_util as SU
 from ilqg_b200 import workloads as W
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 needs_rig = pytest.mark.skipif(not os.path.exists(FM.FAKEMEX), reason="build the fake mex runtime: make -C oracle port")
-PARAMS = {"car": W.CAR_PARAMS, "carhx": W.CARHX_PARAMS, "quad": W.QUAD_PARAMS}
-DIMS = {"car": (4, 2), "carhx": (4, 2), "quad": (12, 4)}
+PARAMS = {"car": W.CAR_PARAMS, "carhx": W.CARHX_PARAMS, "quad": W.QUAD_PARAMS, **{SU.name_of(s): SU.params_of(s) for s in SU.SHAPES}}
+DIMS = {"car": (4, 2), "carhx": (4, 2), "quad": (12, 4), **{SU.name_of(s): s for s in SU.SHAPES}}
 
 
 def gw(kind, problem):
@@ -33,6 +34,9 @@ def point(problem, seed):
     if problem == "quad":
         x = rng.uniform(-0.4, 0.4, nx)
         u = W.QUAD_PARAMS["uh"][0] * (1.0 + rng.uniform(-0.3, 0.3, nu))
+    elif problem.startswith("shape_"):
+        x = rng.uniform(-2.0, 2.0, nx)
+        u = rng.uniform(-0.2, 0.2, nu)         # inside every box: the clamp mode leaves it alone
     else:
         x = np.array([rng.uniform(-2, 2), rng.uniform(-2, 2), rng.uniform(0, 6), rng.uniform(-1, 1)])
         u = np.array([rng.uniform(-0.4, 0.4), rng.uniform(-1.5, 1.5)])
@@ -52,7 +56,7 @@ def fd(fun, z, h=1e-6):
 
 
 @needs_rig
-@pytest.mark.parametrize("problem", ["car", "quad"])
+@pytest.mark.parametrize("problem", ["car", "quad"] + [SU.name_of(s) for s in SU.SHAPES])
 def test_generated_mmex_matches_finite_differences(problem):
     g = gw("cpu", problem)
     p = PARAMS[problem]
@@ -119,7 +123,7 @@ def test_problems_with_folded_constraints_have_no_mmex():
 # ---------------------------------------------------------------------------------------------------- GPU
 @pytest.mark.gpu
 @needs_rig
-@pytest.mark.parametrize("problem", ["car", "carhx", "quad"])
+@pytest.mark.parametrize("problem", ["car", "carhx", "quad"] + [SU.name_of(s) for s in SU.SHAPES])
 def test_gpu_gateway_matches_generated_mmex_in_all_modes(problem):
     cpu, gpu = gw("cpu", problem), gw("b200", problem)
     p = PARAMS[problem]
